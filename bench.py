@@ -2,6 +2,7 @@
 """bench.py -- LogSV Monte Carlo path-steps/sec on B200 (BASELINE.json `metric`), one process per GPU.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--paths P] [--precision fp64|fp32] [--gauss fp32|fp64]
+                    [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P bench.py --gpus N ...
 
 A "step" = one pass of the hot path over one batch of synthetic input: price the whole option chain by Monte Carlo once
@@ -24,7 +25,10 @@ Keys of the JSON line (rank 0):
             profiles/slice_kernel_metrics.json (tools/ncu_summary.py), never from literals here.
 `checks`  : N>1 only -- prices of the p2p exchange vs the NCCL exchange vs ONE GPU running all the paths (SURVEY.md §8d C5: <= 1e-13).
 `extras`  : driver-visible numbers for BASELINE.json configs[0..4] (ms, path-steps/s, error vs the Fourier route / goldens).
-`cpu_baseline` / `--impl reference`: the reference AS SHIPPED (unmodified stochvolmodels 2.2.0 from baseline/_ref, Numba; 1 core =
+`--dump-outputs DIR`: after the timed steps, rank 0 writes what the headline arm's LAST timed step returned -- the chain's 49 MC prices
+            and their standard errors in chain order (float64, DIR/prices.npy and DIR/stds.npy).  Seeds depend only on the step index,
+            so two builds run with the same arguments can be compared output for output.
+`cpu_baseline` / `--impl reference`: the reference AS SHIPPED (unmodified stochvolmodels 2.2.0 in oracle/_ref, Numba; 1 core =
             one call, all cores = one call per worker process) with the oracle's C/OpenMP port beside it, both with effective-core
             accounting (affinity, cgroup quota, measured 1-thread rate and parallel speed-up).
 """
@@ -36,6 +40,7 @@ import os
 import statistics
 import subprocess
 import sys
+import tempfile
 import threading
 import time
 
@@ -149,13 +154,16 @@ def cpu_port_block(chain, params, budget_s: float):
 
 
 def numba_reference_block(budget_s: float, repeat: int, fourier: bool = False, timeout_s: float = 600.0):
-    """run oracle/ref_arm.py (the unmodified reference from baseline/_ref) in a clean subprocess; returns its JSON dict."""
+    """run oracle/ref_arm.py (the unmodified reference in oracle/_ref) in a clean subprocess; returns its JSON dict.  Numba's on-disk
+    cache and Python's bytecode go to a temporary directory / nowhere: the tree may be read-only."""
     cmd = [sys.executable, os.path.join(ROOT, "oracle", "ref_arm.py"), "--budget-s", str(budget_s), "--repeat", str(repeat)]
     if fourier:
         cmd.append("--fourier")
     env = {k: v for k, v in os.environ.items() if k not in ("OMP_NUM_THREADS", "NUMBA_NUM_THREADS")}
     try:
-        out = subprocess.run(cmd, capture_output=True, text=True, timeout=timeout_s, env=env, cwd=ROOT)
+        with tempfile.TemporaryDirectory(prefix="b200sv_numba_") as cache:
+            env.update(NUMBA_CACHE_DIR=cache, PYTHONDONTWRITEBYTECODE="1")
+            out = subprocess.run(cmd, capture_output=True, text=True, timeout=timeout_s, env=env, cwd=ROOT)
         lines = [l for l in out.stdout.splitlines() if l.startswith("{")]
         if out.returncode != 0 or not lines:
             return {"unavailable": f"ref_arm.py rc={out.returncode}: {out.stderr.strip()[-300:]}"}
@@ -191,7 +199,7 @@ def reference_summary(ref: dict):
 
 def run_reference(args, rank, world):
     """--impl reference: the reference's own CPU implementation of the path on the box's host cores, same workload / metric / unit;
-    rank 0 only.  Preferred: the UNMODIFIED reference (baseline/_ref, Numba) on all effective cores, one bounded sample per step;
+    rank 0 only.  Preferred: the UNMODIFIED reference (oracle/_ref, Numba) on all effective cores, one bounded sample per step;
     fallback (reference not installed / numba missing): the oracle's C port."""
     if rank != 0:
         return
@@ -323,10 +331,16 @@ def extra_config4(world, rank, barrier, reduce_max):
 
 
 # ---------------------------------------------------------------------------------------------------------------------------------
+def dump_outputs(path: str, prices: np.ndarray, stds: np.ndarray) -> None:
+    os.makedirs(path, exist_ok=True)
+    np.save(os.path.join(path, "prices.npy"), np.ascontiguousarray(prices, dtype=np.float64))
+    np.save(os.path.join(path, "stds.npy"), np.ascontiguousarray(stds, dtype=np.float64))
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=5)
+    ap.add_argument("--steps", type=int, default=5, help="timed steps (>= 1)")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
     ap.add_argument("--paths", type=float, default=1e8, help="paths per GPU")
@@ -336,7 +350,13 @@ def main():
     ap.add_argument("--no-extras", action="store_true")
     ap.add_argument("--exchange", default="p2p", choices=["p2p", "collective"],
                     help="N>1: per-maturity moment exchange through NVLink peer memory inside the kernels (p2p) or NCCL all-reduce (collective)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the prices and standard errors of the last timed step to DIR/prices.npy and DIR/stds.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be >= 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the outputs of the GPU arm (--impl b200)")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
@@ -463,6 +483,8 @@ def main():
 
     # ---------------- headline: f64 state / f32 draws ----------------
     head = device_arm(args.gauss, args.steps, args.warmup, True)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, head["prices"][0], head["prices"][1])
     e2e_value, prices_api, stds_api = e2e_arm(args.gauss, args.steps, min(args.warmup, 2), args.exchange if world > 1 else None)
     # ---------------- all-fp64 sub-line (fp64 Box-Muller) ----------------
     alt_gauss = "fp64" if args.gauss == "fp32" else "fp32"
@@ -591,7 +613,7 @@ def main():
         if extras:
             line["extras"] = extras
         if not args.no_cpu_baseline and world == 1:
-            # reference as shipped (Numba, unmodified, baseline/_ref) + the C port, both with effective-core accounting
+            # reference as shipped (Numba, unmodified, oracle/_ref) + the C port, both with effective-core accounting
             ref = numba_reference_block(float(os.environ.get("B200SV_BENCH_CPU_BUDGET_S", 8.0)), 1, fourier=True) \
                 if not os.environ.get("B200SV_BENCH_NO_NUMBA") else {"unavailable": "disabled"}
             summary = None if "unavailable" in ref else reference_summary(ref)

@@ -1,11 +1,11 @@
-"""Reference-as-shipped CPU arm: the UNMODIFIED stochvolmodels 2.2.0 (Python + Numba) from ``baseline/_ref``.
+"""Reference-as-shipped CPU arm: the UNMODIFIED stochvolmodels 2.2.0 (Python + Numba) from ``oracle/_ref``.
 
 TEST / MEASUREMENT INFRASTRUCTURE -- imported only by ``bench.py`` (``--impl reference`` and the ``cpu_baseline`` leg) and by
 ``tests/``; never by the product.
 
-``baseline/_ref`` is produced by the committed recipe ``oracle/install_reference.sh`` (``pip install --no-index --no-deps --target
-baseline/_ref`` of a /tmp copy of /root/reference; git-ignored, not gpurun-ignored, so the installed package travels to the GPU box
--- nothing here reads /root/reference at run time).  The three third-party packages the reference imports for plotting / implied
+``oracle/_ref`` is produced by the committed recipe ``oracle/install_reference.sh`` (``pip install --no-index --no-deps --target
+oracle/_ref`` of a temporary copy of the upstream source tree, run by ``build()``; git-ignored -- nothing here reads the source tree at
+run time).  The three third-party packages the reference imports for plotting / implied
 vols (matplotlib, seaborn, vanilla_option_pricers) are absent from the image and replaced by ``MagicMock`` modules: none of them is
 touched by the timed calls (``LogSVPricer.model_mc_price_chain`` logsv_pricer.py:369-427 -> ``logsv_mc_chain_pricer`` :806-867 ->
 ``simulate_logsv_x_vol_terminal`` :950-1047 + ``compute_mc_vars_payoff`` mc_payoffs.py:10-88; ``price_chain`` :345-366).
@@ -25,7 +25,7 @@ from unittest.mock import MagicMock
 import numpy as np
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-REF_DIR = os.path.join(ROOT, "baseline", "_ref")
+REF_DIR = os.path.join(ROOT, "oracle", "_ref")
 _STUBS = ("matplotlib", "matplotlib.pyplot", "matplotlib.backends", "matplotlib.backends.backend_pdf", "matplotlib.lines",
           "matplotlib.ticker", "matplotlib.figure", "matplotlib.axes", "matplotlib.dates", "matplotlib.colors", "seaborn",
           "vanilla_option_pricers", "vanilla_option_pricers.bsm", "vanilla_option_pricers.bachelier")
@@ -34,7 +34,7 @@ _STUBS = ("matplotlib", "matplotlib.pyplot", "matplotlib.backends", "matplotlib.
 def available() -> str:
     """'' when the reference arm can run here, else the one-line reason."""
     if not os.path.isdir(os.path.join(REF_DIR, "stochvolmodels")):
-        return "baseline/_ref/stochvolmodels missing (run oracle/install_reference.sh where /root/reference exists)"
+        return "oracle/_ref/stochvolmodels missing (run oracle/install_reference.sh <StochVolModels source tree>)"
     try:
         import numba  # noqa: F401
     except Exception as e:          # pragma: no cover
@@ -43,7 +43,7 @@ def available() -> str:
 
 
 def import_reference():
-    """import the unmodified reference package from baseline/_ref (stubs for the absent plotting / implied-vol packages)."""
+    """import the unmodified reference package from oracle/_ref (stubs for the absent plotting / implied-vol packages)."""
     for name in _STUBS:
         sys.modules.setdefault(name, MagicMock())
     if REF_DIR not in sys.path:
@@ -51,7 +51,7 @@ def import_reference():
     import stochvolmodels  # noqa: F401
     mod_file = os.path.abspath(sys.modules["stochvolmodels"].__file__)
     if not mod_file.startswith(REF_DIR):
-        raise RuntimeError(f"stochvolmodels resolved to {mod_file}, not to baseline/_ref")
+        raise RuntimeError(f"stochvolmodels resolved to {mod_file}, not to oracle/_ref")
     from stochvolmodels.pricers import logsv_pricer as lp
     from stochvolmodels.pricers import heston_pricer as hp
     from stochvolmodels.data.sample_option_chains import get_btc_test_chain_data

@@ -859,6 +859,49 @@ def params_helpers() -> None:
     print("wrote logsv_params_helpers.npz")
 
 
+def reference_objects() -> None:
+    """The state (``vars()`` after ``__post_init__``) of the reference's own OptionChain / LogSvParams / HestonParams / HawkesJDParams
+    objects that tests/test_reference_ducktyping.py hands to the B200 pricers, and the members of its VariableType enum
+    -> reference_objects.npz.  Key ``<obj>__fields`` lists the attributes in order; ``<obj>__<attr>`` holds a value, ``<obj>__<attr>__<i>``
+    the i-th array of a list; an attribute with neither is None.  ``<obj>@<method>`` records what the reference's methods that the pricers
+    call returned: get_vol_backbone_eta at the chain's maturities ([taus, etas]) and the keys of to_dict().
+    python tests/golden/make_golden.py --only-objects"""
+    _import_reference()
+    from stochvolmodels.data.option_chain import OptionChain
+    from stochvolmodels.pricers.hawkes_jd_pricer import HawkesJDParams
+    from stochvolmodels.pricers.heston_pricer import HestonParams
+    from stochvolmodels.pricers.logsv.logsv_params import LogSvParams
+    from stochvolmodels.utils.config import VariableType
+    hawkes = dict(sigma=0.4, mean_p=0.04, mean_m=-0.05, theta_p=6.0, lambda_p=7.0, kappa_p=20.0, beta1_p=30.0, beta2_p=-25.0)
+    objects = dict(
+        chain=OptionChain(ttms=np.array([0.1, 0.3]), forwards=np.array([1.0, 1.02]), discfactors=np.array([1.0, 0.99]), ids=np.array(["a", "b"]),
+                          strikes_ttms=[np.array([0.9, 1.0, 1.1]), np.array([0.8, 1.2])],
+                          optiontypes_ttms=[np.array(["P", "C", "C"]), np.array(["P", "C"])]),
+        logsv=LogSvParams(sigma0=0.9, theta=1.0, kappa1=4.0, kappa2=3.0, beta=0.3, volvol=1.5),
+        logsv_params5=LogSvParams(sigma0=0.9, theta=0.8, kappa1=4.0, kappa2=None, beta=0.3, volvol=1.5),
+        heston=HestonParams(v0=0.05, theta=0.06, kappa=3.0, rho=-0.4, volvol=0.7),
+        hawkes=HawkesJDParams(**hawkes),
+        hawkes_gamma=HawkesJDParams(risk_premia_gamma=0.3, **hawkes))
+    out = dict(variable_type_names=np.array([m.name for m in VariableType]), variable_type_values=np.array([m.value for m in VariableType]))
+    for name, obj in objects.items():
+        out[f"{name}__fields"] = np.array(list(vars(obj)))
+        for attr, v in vars(obj).items():
+            if isinstance(v, (list, tuple)):
+                for i, a in enumerate(v):
+                    out[f"{name}__{attr}__{i}"] = np.asarray(a)
+            elif v is not None:
+                out[f"{name}__{attr}"] = np.asarray(v)
+        if isinstance(obj, LogSvParams):
+            taus = objects["chain"].ttms
+            etas = np.array([obj.get_vol_backbone_eta(tau=t) for t in taus], dtype=float)
+            assert np.array_equal(etas, obj.get_vol_backbone_etas(ttms=taus))
+            out[f"{name}@get_vol_backbone_eta"] = np.stack([taus, etas])
+        if isinstance(obj, HawkesJDParams):
+            out[f"{name}@to_dict"] = np.array(list(obj.to_dict()))
+    np.savez(os.path.join(OUT, "reference_objects.npz"), **out)
+    print("wrote reference_objects.npz")
+
+
 def _chain(ttms, fw, df, K, T):
     from stochvolmodels.data.option_chain import OptionChain
     from numba.typed import List
@@ -867,6 +910,9 @@ def _chain(ttms, fw, df, K, T):
 
 
 if __name__ == "__main__":
+    if "--only-objects" in sys.argv:
+        reference_objects()
+        sys.exit(0)
     if "--only-hawkes-fourier" in sys.argv:
         hawkes_fourier()
         sys.exit(0)

@@ -44,10 +44,10 @@ def test_reference_arm_port_fallback_json_line_and_core_count():
 
 
 def test_reference_arm_runs_the_unmodified_numba_reference_when_installed():
-    """baseline/_ref (oracle/install_reference.sh) present: the arm is the reference as shipped -- Numba, one process per core"""
-    if not os.path.isdir(os.path.join(ROOT, "baseline", "_ref", "stochvolmodels")):
+    """oracle/_ref (oracle/install_reference.sh) present: the arm is the reference as shipped -- Numba, one process per core"""
+    if not os.path.isdir(os.path.join(ROOT, "oracle", "_ref", "stochvolmodels")):
         import pytest
-        pytest.skip("baseline/_ref not installed in this checkout")
+        pytest.skip("oracle/_ref not installed in this checkout")
     r = _run(["--impl", "reference", "--steps", "1", "--warmup", "0", "--gpus", "2"], {"OMP_NUM_THREADS": "1", "RANK": "0", "WORLD_SIZE": "2",
                                                                                          "B200SV_BENCH_CPU_BUDGET_S": "1"}, timeout=600)
     d = _check_line(r)

@@ -127,7 +127,7 @@ def test_gather_timeout_is_an_error_not_a_silent_nan(cuda_lib):
 def test_two_gpu_exchange_vs_nccl_and_single_gpu(cuda_lib):
     import torch
     if torch.cuda.device_count() < 2:
-        pytest.skip("needs 2 GPUs (the round driver's N>1 runs and `gpurun --gpus 2` cover it)")
+        pytest.skip("needs 2 GPUs: the peer-memory exchange is between two devices")
     cmd = [sys.executable, "-m", "torch.distributed.run", "--nnodes=1", "--nproc-per-node", "2", "--master-addr", "127.0.0.1",
            "--master-port", "29533", os.path.join(ROOT, "tools", "check_multi_gpu.py")]
     r = subprocess.run(cmd, capture_output=True, text=True, timeout=600)

@@ -1,7 +1,7 @@
 """GPU: the REFERENCE'S OWN test files, run against this package as a drop-in (tools/run_reference_tests.py).
 
-The unmodified stochvolmodels wheel that oracle/install_reference.sh installs into git-ignored baseline/_ref ships its test-suite; it travels to
-the GPU box with the snapshot.  The tool aliases the module paths those tests import to stochvolmodels_b200 and runs them; here the outcome is
+The unmodified stochvolmodels wheel that oracle/install_reference.sh installs into git-ignored oracle/_ref (run by build()
+where the upstream source tree is readable) ships its test-suite.  The tool aliases the module paths those tests import to stochvolmodels_b200 and runs them; here the outcome is
 pinned: the files that only touch the paths of SURVEY.md section 8 must pass completely, and the total must not regress."""
 import os
 import re
@@ -11,7 +11,7 @@ import sys
 import pytest
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-REF_TESTS = os.path.join(ROOT, "baseline", "_ref", "stochvolmodels", "tests")
+REF_TESTS = os.path.join(ROOT, "oracle", "_ref", "stochvolmodels", "tests")
 pytestmark = pytest.mark.gpu
 # substrings of the reference tests that need something this package does not rebuild (profiles/r02_reference_tests.txt lists the causes)
 OUT_OF_SCOPE = ("approximate_logsv", "rough_kernel_approximation", "affine_grid_solvers_preserve_transform_roots", "all_bundled_sample_chains", "swaption_chain", "futures_chain", "rough_logsv_pricer_pricing_regression",
@@ -33,7 +33,7 @@ def _run(*stems):
     return counts, per_file, out
 
 
-@pytest.mark.skipif(not os.path.isdir(REF_TESTS), reason="baseline/_ref (the reference wheel with its tests) is not installed")
+@pytest.mark.skipif(not os.path.isdir(REF_TESTS), reason="oracle/_ref (the reference wheel with its tests) is not installed")
 def test_the_references_own_tests_pass_against_this_package(cuda_lib):
     counts, per_file, out = _run()
     tail = out[-3000:]

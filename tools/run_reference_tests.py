@@ -1,8 +1,8 @@
-"""Run the REFERENCE'S OWN test files against this package as a drop-in (GPU box: needs CUDA and baseline/_ref).
+"""Run the REFERENCE'S OWN test files against this package as a drop-in (needs CUDA and oracle/_ref).
 
     python tools/run_reference_tests.py [test_file_stem ...]          # default: the files that touch SURVEY.md section 8's paths
 
-The unmodified stochvolmodels 2.2.0 wheel that oracle/install_reference.sh puts into baseline/_ref ships its test-suite
+The unmodified stochvolmodels 2.2.0 wheel that oracle/install_reference.sh puts into oracle/_ref ships its test-suite
 (stochvolmodels/tests).  This tool aliases the module paths those tests import (``stochvolmodels.pricers.logsv_pricer`` ...) to the modules
 of stochvolmodels_b200 in ``sys.modules`` -- no file of the reference is imported except its test files -- gives plain functions the
 ``py_func`` attribute the tests reach for on Numba dispatchers, and runs pytest on copies of the test files in a temporary directory.
@@ -18,7 +18,7 @@ import types
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
-REF_TESTS = os.path.join(ROOT, "baseline", "_ref", "stochvolmodels", "tests")
+REF_TESTS = os.path.join(ROOT, "oracle", "_ref", "stochvolmodels", "tests")
 
 # reference module path -> module(s) of this package whose public names it exposes (later entries fill names the earlier ones lack)
 ALIASES = {
@@ -142,7 +142,7 @@ def install_aliases():
 def main(argv):
     import pytest
     if not os.path.isdir(REF_TESTS):
-        print(f"{REF_TESTS} is missing: run oracle/install_reference.sh (needs /root/reference) first")
+        print(f"{REF_TESTS} is missing: run oracle/install_reference.sh <StochVolModels source tree> first")
         return 2
     install_aliases()
     files = argv or DEFAULT_FILES
