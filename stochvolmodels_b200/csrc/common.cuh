@@ -99,5 +99,47 @@ inline void ensure_pool_threshold() {
   done_for = dev;
 }
 
+// Kernels launched by the calling thread (b200sv_launch_count).  Defined once in mc_kernels.cu.
+long long& launch_count();
+
+// Check a kernel launch (a cooperative launch passes its own result): an error becomes -2, a launch is counted.
+inline int launched(const char* what, cudaError_t e = cudaGetLastError()) {
+  if (e != cudaSuccess) return fail(-2, std::string(what) + ": " + cudaGetErrorString(e));
+  ++launch_count();
+  return 0;
+}
+
+// A stream-ordered device temporary of n T's, freed on its stream when it goes out of scope.
+template <typename T>
+struct DevBuf {
+  T* p = nullptr;
+  cudaStream_t st;
+  explicit DevBuf(cudaStream_t s) : st(s) {}
+  DevBuf(const DevBuf&) = delete;
+  DevBuf& operator=(const DevBuf&) = delete;
+  ~DevBuf() {
+    if (p) cudaFreeAsync(p, st);
+  }
+  cudaError_t alloc(size_t n) { return cudaMallocAsync((void**)&p, sizeof(T) * (n ? n : 1), st); }
+  // alloc(n), then copy n T's from host memory
+  cudaError_t upload(const void* src, size_t n) {
+    const cudaError_t e = alloc(n);
+    return e != cudaSuccess || n == 0 ? e : cudaMemcpyAsync(p, src, sizeof(T) * n, cudaMemcpyHostToDevice, st);
+  }
+};
+
+// Body of a host-level entry point: body(stream) runs on the calling thread's stream (b200sv_set_stream) and declares its DevBufs
+// inside, so they are freed when it returns.  The stream is then drained once on every path -- no copy into the caller's (possibly
+// pinned) memory is in flight after the call -- and the first error is returned.
+template <typename Body>
+inline int host_call(Body&& body) {
+  const cudaStream_t st = current_stream();
+  ensure_pool_threshold();
+  int rc = body(st);
+  const cudaError_t e = cudaStreamSynchronize(st);
+  if (rc == 0 && e != cudaSuccess) rc = fail(-2, std::string("cudaStreamSynchronize: ") + cudaGetErrorString(e));
+  return rc;
+}
+
 
 }  // namespace b200sv

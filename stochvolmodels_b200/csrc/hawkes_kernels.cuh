@@ -251,11 +251,15 @@ __global__ void hawkes_device_draws_kernel(unsigned long long seed, unsigned lon
   }
 }
 
+static int check_hawkes_flags(int flags) {
+  const int g = gauss_mode(flags);
+  return g == kGaussF32 || g == kGaussF64 ? 0 : fail(-1, "invalid argument: gauss flags");
+}
+
 static int launch_hawkes_slice(double* x, double* lp, double* lm, long long n, long long path_offset, int init, const b200sv_hawkes_params& p,
                                int nsteps, double dt, int slice_index, double forward, uint64_t seed, int flags, double* moments_out,
                                cudaStream_t st, P2pCtx* p2p = nullptr) {
-  const int g = gauss_mode(flags);
-  if (g != kGaussF32 && g != kGaussF64) return fail(-1, "invalid argument: gauss flags");
+  if (int rc = check_hawkes_flags(flags)) return rc;
   HawkesSliceArgs a;
   a.x = x;
   a.lam_p = lp;
@@ -271,81 +275,47 @@ static int launch_hawkes_slice(double* x, double* lp, double* lm, long long n, l
   a.forward = forward;
   const HawkesConsts c = make_hawkes_consts(p, dt);
   Grid grid = persistent_grid(hawkes_slice_kernel<kGaussF32>, kThreads, n);
-  double* partials = nullptr;
+  DevBuf<double> partials(st);
   ensure_pool_threshold();
-  B200SV_CUDA(cudaMallocAsync(&partials, sizeof(double) * 2 * grid.blocks, st));
-  a.partials = partials;
-  if (g == kGaussF64)
+  B200SV_CUDA(partials.alloc(2 * (size_t)grid.blocks));
+  a.partials = partials.p;
+  if (gauss_mode(flags) == kGaussF64)
     hawkes_slice_kernel<kGaussF64><<<grid.blocks, grid.threads, 0, st>>>(a, c);
   else
     hawkes_slice_kernel<kGaussF32><<<grid.blocks, grid.threads, 0, st>>>(a, c);
-  if (int rc = check_launch("hawkes_slice_kernel")) return rc;
-  reduce_partials_kernel<<<1, 64, 0, st>>>(partials, grid.blocks, 2, 2, moments_out, make_publish(p2p, st));   // exchange #1 (producer)
-  if (int rc = check_launch("reduce_partials_kernel")) return rc;
-  B200SV_CUDA(cudaFreeAsync(partials, st));
-  return 0;
+  if (int rc = launched("hawkes_slice_kernel")) return rc;
+  reduce_partials_kernel<<<1, 64, 0, st>>>(partials.p, grid.blocks, 2, 2, moments_out, make_publish(p2p, st));   // exchange #1 (producer)
+  return launched("reduce_partials_kernel");
 }
 
 constexpr int kHawkesStepsPerYear = 5 * 360;     // hawkes_jd_pricer.py:752
 
 static int hawkes_chain_host(const b200sv_hawkes_params* p, int M, const double* ttms, const double* forwards, const double* discfactors,
                              const int* offsets, const double* strikes, const int8_t* types, long long nb_path, int variable_type, uint64_t seed,
-                             int flags, double* prices_out, double* stderr_out, double* state_out /* [3][nb_path] or NULL */) {
+                             int flags, double* prices_out, double* stderr_out) {
   B200SV_REQUIRE(nb_path >= 1, "nb_path must be >= 1");
   B200SV_REQUIRE(!(flags & B200SV_STATE_F32), "the Hawkes route is float64 only");
   if (int rc = validate_chain(M, ttms, offsets, types, variable_type)) return rc;
-  const int Jtot = offsets[M] - offsets[0], Jalloc = std::max(Jtot, 1);
-  cudaStream_t st = current_stream();
-  ensure_pool_threshold();
-  double *d = nullptr, *d_strikes = nullptr, *d_out = nullptr, *d_mom = nullptr, *d_sums = nullptr;
-  int8_t* d_types = nullptr;
+  if (int rc = check_hawkes_flags(flags)) return rc;
   const size_t N = (size_t)nb_path;
-  B200SV_CUDA(cudaMallocAsync(&d, sizeof(double) * 3 * N, st));
-  B200SV_CUDA(cudaMallocAsync(&d_strikes, sizeof(double) * Jalloc, st));
-  B200SV_CUDA(cudaMallocAsync(&d_types, Jalloc, st));
-  B200SV_CUDA(cudaMallocAsync(&d_out, sizeof(double) * 2 * Jalloc, st));
-  B200SV_CUDA(cudaMallocAsync(&d_mom, sizeof(double) * 2, st));
-  B200SV_CUDA(cudaMallocAsync(&d_sums, sizeof(double) * 3 * Jalloc, st));
-  if (Jtot > 0) {
-    B200SV_CUDA(cudaMemcpyAsync(d_strikes, strikes + offsets[0], sizeof(double) * Jtot, cudaMemcpyHostToDevice, st));
-    B200SV_CUDA(cudaMemcpyAsync(d_types, types + offsets[0], Jtot, cudaMemcpyHostToDevice, st));
-  }
-  int rc = 0;
-  double t0 = 0.0;
-  for (int m = 0; m < M && rc == 0; ++m) {
-    int S;
-    double dt;
-    time_grid(ttms[m] - t0, kHawkesStepsPerYear, &S, &dt);
-    t0 = ttms[m];
-    rc = launch_hawkes_slice(d, d + N, d + 2 * N, nb_path, 0, m == 0, *p, S, dt, m, forwards[m], seed, flags, d_mom, st);
-    if (rc) break;
-    const int J = offsets[m + 1] - offsets[m], jo = offsets[m] - offsets[0];
-    if (J == 0) continue;
-    // compute_mc_vars_payoff(x0=x0, sigma0=x0, qvar0=x0, ...) (:703): the log-return array stands in for every argument
-    rc = launch_payoff_t<double>(d, d, nb_path, ttms[m], forwards[m], d_strikes + jo, d_types + jo, J, variable_type, payoff_kinds(types + offsets[m], J),
-                                 d_mom, d_sums, st);
-    if (rc) break;
-    payoff_finalize_kernel<<<(J + 127) / 128, 128, 0, st>>>(d_sums, J, discfactors[m], (double)nb_path, d_out + jo, d_out + Jalloc + jo, P2pGather{});
-    rc = check_launch("payoff_finalize_kernel");
-  }
-  if (rc == 0 && Jtot > 0) {
-    cudaError_t e = cudaMemcpyAsync(prices_out, d_out, sizeof(double) * Jtot, cudaMemcpyDeviceToHost, st);
-    if (e == cudaSuccess) e = cudaMemcpyAsync(stderr_out, d_out + Jalloc, sizeof(double) * Jtot, cudaMemcpyDeviceToHost, st);
-    if (e != cudaSuccess) rc = fail(-2, std::string("D2H: ") + cudaGetErrorString(e));
-  }
-  if (rc == 0 && state_out) {
-    cudaError_t e = cudaMemcpyAsync(state_out, d, sizeof(double) * 3 * N, cudaMemcpyDeviceToHost, st);
-    if (e != cudaSuccess) rc = fail(-2, std::string("D2H: ") + cudaGetErrorString(e));
-  }
-  cudaFreeAsync(d, st);
-  cudaFreeAsync(d_strikes, st);
-  cudaFreeAsync(d_types, st);
-  cudaFreeAsync(d_out, st);
-  cudaFreeAsync(d_mom, st);
-  cudaFreeAsync(d_sums, st);
-  cudaError_t e = cudaStreamSynchronize(st);
-  if (rc == 0 && e != cudaSuccess) rc = fail(-2, std::string("sync: ") + cudaGetErrorString(e));
-  return rc;
+  return host_call([&](cudaStream_t st) {
+    DevBuf<double> d(st);
+    ChainPayoffs pay(st, M, ttms, forwards, discfactors, offsets, types, variable_type, 1, false);
+    B200SV_CUDA(d.alloc(3 * N));
+    if (int rc = pay.alloc(strikes)) return rc;
+    double t0 = 0.0;
+    for (int m = 0; m < M; ++m) {
+      int S;
+      double dt;
+      time_grid(ttms[m] - t0, kHawkesStepsPerYear, &S, &dt);
+      t0 = ttms[m];
+      if (int rc = launch_hawkes_slice(d.p, d.p + N, d.p + 2 * N, nb_path, 0, m == 0, *p, S, dt, m, forwards[m], seed, flags, pay.d_mom.p, st))
+        return rc;
+      // compute_mc_vars_payoff(x0=x0, sigma0=x0, qvar0=x0, ...) (:703): the log-return array stands in for every argument
+      if (int rc = pay.run(0, m, d.p, d.p, nb_path, false, (double)nb_path, st)) return rc;
+    }
+    return pay.copy_back(prices_out, stderr_out, nullptr, st);
+  });
 }
 
 }  // namespace b200sv

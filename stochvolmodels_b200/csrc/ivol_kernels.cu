@@ -14,8 +14,6 @@
 #include "common.cuh"
 #include "black.cuh"
 
-extern "C" void b200sv_internal_count_launch(void);
-
 namespace b200sv {
 
 struct QuoteSpec {
@@ -46,20 +44,14 @@ extern "C" int b200sv_bsm_implied_vols(int M, const double* ttms, const double* 
       if (types[j] < 0 || types[j] > 3) return fail(-3, "unknown option payoff code");
       q[j - offsets[0]] = QuoteSpec{forwards[m], strikes[j], ttms[m], discfactors[m], prices[j - offsets[0]], (int)types[j]};
     }
-  cudaStream_t st = current_stream();
-  ensure_pool_threshold();
-  QuoteSpec* dq = nullptr;
-  double* dv = nullptr;
-  B200SV_CUDA(cudaMallocAsync(&dq, sizeof(QuoteSpec) * n, st));
-  B200SV_CUDA(cudaMallocAsync(&dv, sizeof(double) * n, st));
-  B200SV_CUDA(cudaMemcpyAsync(dq, q.data(), sizeof(QuoteSpec) * n, cudaMemcpyHostToDevice, st));
-  black_ivol_kernel<<<(n + 63) / 64, 64, 0, st>>>(dq, n, dv);
-  cudaError_t e = cudaGetLastError();
-  if (e != cudaSuccess) return fail(-2, std::string("black_ivol_kernel: ") + cudaGetErrorString(e));
-  b200sv_internal_count_launch();
-  B200SV_CUDA(cudaMemcpyAsync(ivols_out, dv, sizeof(double) * n, cudaMemcpyDeviceToHost, st));
-  cudaFreeAsync(dq, st);
-  cudaFreeAsync(dv, st);
-  B200SV_CUDA(cudaStreamSynchronize(st));
-  return 0;
+  return host_call([&](cudaStream_t st) {
+    DevBuf<QuoteSpec> dq(st);
+    DevBuf<double> dv(st);
+    B200SV_CUDA(dq.upload(q.data(), n));
+    B200SV_CUDA(dv.alloc(n));
+    black_ivol_kernel<<<(n + 63) / 64, 64, 0, st>>>(dq.p, n, dv.p);
+    if (int rc = launched("black_ivol_kernel")) return rc;
+    B200SV_CUDA(cudaMemcpyAsync(ivols_out, dv.p, sizeof(double) * n, cudaMemcpyDeviceToHost, st));
+    return 0;
+  });
 }

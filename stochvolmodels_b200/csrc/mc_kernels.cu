@@ -34,10 +34,13 @@
 
 namespace b200sv {
 
-static thread_local long long g_launches = 0;
 cudaStream_t& current_stream_ref() {
   static thread_local cudaStream_t st = nullptr;
   return st;
+}
+long long& launch_count() {
+  static thread_local long long n = 0;
+  return n;
 }
 constexpr int kThreads = 256;
 #ifndef B200SV_SLICE_PREFETCH
@@ -996,23 +999,39 @@ static P2pGather make_gather(P2pCtx* c) {
   return g;
 }
 
-static int check_launch(const char* what) {
-  cudaError_t e = cudaGetLastError();
-  if (e != cudaSuccess) return fail(-2, std::string(what) + ": " + cudaGetErrorString(e));
-  ++g_launches;
-  return 0;
-}
-
 // int(ttm * n) + 1 and dt = linspace(0, ttm, S+1)[1] - [0] (utils/funcs.py:44-47; numpy linspace: step = ttm / S, y[1] = 1*step)
 static void time_grid(double ttm, int n_per_year, int* S, double* dt) {
   *S = (int)(ttm * (double)n_per_year) + 1;
   *dt = (*S == 1) ? ttm : ttm / (double)(*S);   // linspace sets the LAST point to `stop` exactly; with S == 1 y[1] is that point
 }
 
+// model -> (path, constants) of the slice and chain kernels: 0 LogSV, 1 Heston floor-Euler, 2 Heston QE
+template <int MODEL>
+struct ChainModel;
+template <>
+struct ChainModel<0> {
+  template <typename Real>
+  using Path = LogsvPath<Real>;
+  using Consts = LogsvConsts;
+};
+template <>
+struct ChainModel<1> {
+  template <typename Real>
+  using Path = HestonPath<Real, false>;
+  using Consts = HestonConsts;
+};
+template <>
+struct ChainModel<2> {
+  template <typename Real>
+  using Path = HestonPath<Real, true>;
+  using Consts = HestonConsts;
+};
+
 template <int MODEL, typename Real, int G64>
 static int launch_slice_t(void* x, void* v, void* q, long long n, long long path_offset, int init, double v_init, int nsteps,
-                          int slice_index, double forward, uint64_t seed, const LogsvConsts* lc, const HestonConsts* hc,
-                          double* moments_out, cudaStream_t st, P2pCtx* p2p = nullptr) {
+                          int slice_index, double forward, uint64_t seed, const typename ChainModel<MODEL>::Consts& c,
+                          double* moments_out, cudaStream_t st, P2pCtx* p2p) {
+  const auto kernel = mc_slice_kernel<typename ChainModel<MODEL>::template Path<Real>, typename ChainModel<MODEL>::Consts, Real, G64>;
   SliceArgs<Real> a;
   a.x = (Real*)x;
   a.v = (Real*)v;
@@ -1025,41 +1044,26 @@ static int launch_slice_t(void* x, void* v, void* q, long long n, long long path
   a.slice = (unsigned int)slice_index;
   a.seed = seed;
   a.forward = forward;
-  const bool qe = MODEL == 1 && hc->qe;
-  Grid g;
-  if constexpr (MODEL == 0)
-    g = persistent_grid(mc_slice_kernel<LogsvPath<Real>, LogsvConsts, Real, G64>, kSliceThreads, n);
-  else if (qe)
-    g = persistent_grid(mc_slice_kernel<HestonPath<Real, true>, HestonConsts, Real, G64>, kSliceThreads, n);
-  else
-    g = persistent_grid(mc_slice_kernel<HestonPath<Real, false>, HestonConsts, Real, G64>, kSliceThreads, n);
+  Grid g = persistent_grid(kernel, kSliceThreads, n);
   size_t dyn_smem = 0;
 #ifdef B200SV_TUNING   // occupancy sweep for profiles/: cap resident CTAs per SM with dynamic shared memory (tuning builds only)
   if (const char* e = getenv("B200SV_DEBUG_BLOCKS_PER_SM")) {
     const int bps = atoi(e);
     if (bps > 0) {
       dyn_smem = (size_t)(200 * 1024) / bps;
-      if constexpr (MODEL == 0)
-        cudaFuncSetAttribute(mc_slice_kernel<LogsvPath<Real>, LogsvConsts, Real, G64>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)dyn_smem);
+      if constexpr (MODEL == 0) cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)dyn_smem);
       g.blocks = (int)std::min<long long>((long long)148 * bps, (n + kSliceThreads - 1) / kSliceThreads);
     }
   }
 #endif
-  double* partials = nullptr;
+  DevBuf<double> partials(st);
   ensure_pool_threshold();      // device-level callers too: a pool that trims at every synchronisation stalls the whole node (DESIGN.md 5)
-  B200SV_CUDA(cudaMallocAsync(&partials, sizeof(double) * 2 * g.blocks, st));
-  a.partials = partials;
-  if constexpr (MODEL == 0)
-    mc_slice_kernel<LogsvPath<Real>, LogsvConsts, Real, G64><<<g.blocks, g.threads, dyn_smem, st>>>(a, *lc);
-  else if (qe)
-    mc_slice_kernel<HestonPath<Real, true>, HestonConsts, Real, G64><<<g.blocks, g.threads, dyn_smem, st>>>(a, *hc);
-  else
-    mc_slice_kernel<HestonPath<Real, false>, HestonConsts, Real, G64><<<g.blocks, g.threads, dyn_smem, st>>>(a, *hc);
-  if (int rc = check_launch("mc_slice_kernel")) return rc;
-  reduce_partials_kernel<<<1, 64, 0, st>>>(partials, g.blocks, 2, 2, moments_out, make_publish(p2p, st));   // exchange #1 (producer)
-  if (int rc = check_launch("reduce_partials_kernel")) return rc;
-  B200SV_CUDA(cudaFreeAsync(partials, st));
-  return 0;
+  B200SV_CUDA(partials.alloc(2 * (size_t)g.blocks));
+  a.partials = partials.p;
+  kernel<<<g.blocks, g.threads, dyn_smem, st>>>(a, c);
+  if (int rc = launched("mc_slice_kernel")) return rc;
+  reduce_partials_kernel<<<1, 64, 0, st>>>(partials.p, g.blocks, 2, 2, moments_out, make_publish(p2p, st));   // exchange #1 (producer)
+  return launched("reduce_partials_kernel");
 }
 
 // B200SV_GAUSS_* bits -> GaussMode (philox.cuh); -1 = contradictory
@@ -1069,21 +1073,31 @@ static int gauss_mode(int flags) {
   return paired ? kGaussF64Paired : (g64 ? kGaussF64 : kGaussF32);
 }
 
-template <int MODEL>
-static int launch_slice(void* x, void* v, void* q, long long n, long long path_offset, int init, double v_init, int nsteps,
-                        int slice_index, double forward, uint64_t seed, int flags, const LogsvConsts* lc, const HestonConsts* hc,
-                        double* moments_out, cudaStream_t st, P2pCtx* p2p = nullptr) {
-  const bool f32 = flags & B200SV_STATE_F32;
+// the state / Gaussian flag combinations the slice kernels are built for
+static int check_slice_flags(int flags) {
   const int g = gauss_mode(flags);
   if (g < 0) return fail(-1, "invalid argument: B200SV_GAUSS_F64 and B200SV_GAUSS_F64_PAIRED are mutually exclusive");
+  if ((flags & B200SV_STATE_F32) && g == kGaussF64Paired) return fail(-1, "invalid argument: the paired Gaussian check mode needs fp64 state");
+  return 0;
+}
+
+// MODEL 0 = LogSV, 1 = Heston (the QE scheme, c.qe, runs model 2)
+template <int MODEL>
+static int launch_slice(void* x, void* v, void* q, long long n, long long path_offset, int init, double v_init, int nsteps,
+                        int slice_index, double forward, uint64_t seed, int flags, const typename ChainModel<MODEL>::Consts& c,
+                        double* moments_out, cudaStream_t st, P2pCtx* p2p = nullptr) {
+  if constexpr (MODEL == 1)
+    if (c.qe) return launch_slice<2>(x, v, q, n, path_offset, init, v_init, nsteps, slice_index, forward, seed, flags, c, moments_out, st, p2p);
+  if (int rc = check_slice_flags(flags)) return rc;
+  const bool f32 = flags & B200SV_STATE_F32;
+  const int g = gauss_mode(flags);
 #define B200SV_SLICE_CASE(REAL, G) \
-  return launch_slice_t<MODEL, REAL, G>(x, v, q, n, path_offset, init, v_init, nsteps, slice_index, forward, seed, lc, hc, moments_out, st, p2p)
+  return launch_slice_t<MODEL, REAL, G>(x, v, q, n, path_offset, init, v_init, nsteps, slice_index, forward, seed, c, moments_out, st, p2p)
   if (!f32 && g == kGaussF32) B200SV_SLICE_CASE(double, kGaussF32);
   if (!f32 && g == kGaussF64) B200SV_SLICE_CASE(double, kGaussF64);
   if (!f32 && g == kGaussF64Paired) B200SV_SLICE_CASE(double, kGaussF64Paired);
   if (f32 && g == kGaussF32) B200SV_SLICE_CASE(float, kGaussF32);
-  if (f32 && g == kGaussF64) B200SV_SLICE_CASE(float, kGaussF64);
-  return fail(-1, "invalid argument: the paired Gaussian check mode needs fp64 state");
+  B200SV_SLICE_CASE(float, kGaussF64);
 #undef B200SV_SLICE_CASE
 }
 
@@ -1099,20 +1113,18 @@ static int launch_payoff_t(const void* x, const void* q, long long n, double ttm
   const bool vanilla = kinds == 1;
   Grid g = vanilla ? persistent_grid(payoff_vanilla_kernel<Real>, kThreads, n, kPayoffUnroll) : persistent_grid(payoff_kernel<Real>, kThreads, n);
   g.blocks = std::max(1, g.blocks / chunks);
-  double* partials = nullptr;
+  DevBuf<double> partials(st);
   ensure_pool_threshold();
-  B200SV_CUDA(cudaMallocAsync(&partials, sizeof(double) * (size_t)Kpad * g.blocks, st));
+  B200SV_CUDA(partials.alloc((size_t)Kpad * g.blocks));
   if (vanilla)
     payoff_vanilla_kernel<Real><<<dim3(g.blocks, chunks), g.threads, 0, st>>>((const Real*)x, (const Real*)q, n, ttm, forward, strikes,
-                                                                                types, J, variable_type, moments, partials, Kpad, gat);
+                                                                                types, J, variable_type, moments, partials.p, Kpad, gat);
   else
     payoff_kernel<Real><<<dim3(g.blocks, chunks), g.threads, 0, st>>>((const Real*)x, (const Real*)q, n, ttm, forward, strikes,
-                                                                        types, J, variable_type, moments, partials, Kpad, gat);
-  if (int rc = check_launch("payoff_kernel")) return rc;
-  reduce_partials_kernel<<<1, 256, 0, st>>>(partials, g.blocks, Kpad, 3 * J, sums_out, make_publish(p2p, st));   // exchange #2 (producer)
-  if (int rc = check_launch("reduce_partials_kernel")) return rc;
-  B200SV_CUDA(cudaFreeAsync(partials, st));
-  return 0;
+                                                                        types, J, variable_type, moments, partials.p, Kpad, gat);
+  if (int rc = launched("payoff_kernel")) return rc;
+  reduce_partials_kernel<<<1, 256, 0, st>>>(partials.p, g.blocks, Kpad, 3 * J, sums_out, make_publish(p2p, st));   // exchange #2 (producer)
+  return launched("reduce_partials_kernel");
 }
 
 static int payoff_kinds(const int8_t* types, int J) {
@@ -1136,43 +1148,77 @@ static int validate_chain(int M, const double* ttms, const int* offsets, const i
   return 0;
 }
 
-// one cooperative launch for the whole chain of one parameter set (fp64 state); buffers come from the caller
-template <int MODEL, int GAUSS>
-static int launch_chain_coop_g(const CoopArgs& args, const void* d_specs, int grid_blocks, cudaStream_t st) {
-  CoopArgs a = args;
-  const void* sp = d_specs;
-  void* kargs[] = {(void*)&a, (void*)&sp};
-  cudaError_t e;
-  if constexpr (MODEL == 0)
-    e = cudaLaunchCooperativeKernel((void*)mc_chain_coop_kernel<LogsvPath<double>, LogsvConsts, GAUSS>, dim3(grid_blocks), dim3(kSliceThreads), kargs, 0, st);
-  else if constexpr (MODEL == 1)
-    e = cudaLaunchCooperativeKernel((void*)mc_chain_coop_kernel<HestonPath<double, false>, HestonConsts, GAUSS>, dim3(grid_blocks), dim3(kSliceThreads), kargs, 0, st);
-  else
-    e = cudaLaunchCooperativeKernel((void*)mc_chain_coop_kernel<HestonPath<double, true>, HestonConsts, GAUSS>, dim3(grid_blocks), dim3(kSliceThreads), kargs, 0, st);
-  if (e != cudaSuccess) return fail(-2, std::string("mc_chain_coop_kernel: ") + cudaGetErrorString(e));
-  ++g_launches;
+// The payoff stage of the host-level MC chain drivers: the chain's strikes and types on the device, the moment and sum scratch, and B sets
+// of outputs [prices | std errors | implied vols if asked for] of Jalloc values each, written per (set, maturity) and copied back once.
+struct ChainPayoffs {
+  const double *ttms, *forwards, *discfactors;
+  const int* offsets;
+  const int8_t* types;
+  int variable_type, B, Jtot, Jalloc, nout;
+  DevBuf<double> d_strikes, d_mom, d_sums, d_out;
+  DevBuf<int8_t> d_types;
+
+  ChainPayoffs(cudaStream_t st, int M, const double* ttms, const double* forwards, const double* discfactors, const int* offsets,
+               const int8_t* types, int variable_type, int B, bool ivols)
+      : ttms(ttms), forwards(forwards), discfactors(discfactors), offsets(offsets), types(types), variable_type(variable_type), B(B),
+        Jtot(offsets[M] - offsets[0]), Jalloc(std::max(Jtot, 1)), nout(ivols ? 3 : 2), d_strikes(st), d_mom(st), d_sums(st), d_out(st),
+        d_types(st) {}
+
+  int alloc(const double* strikes) {
+    B200SV_CUDA(d_strikes.upload(strikes + offsets[0], Jtot));
+    B200SV_CUDA(d_types.upload(types + offsets[0], Jtot));
+    B200SV_CUDA(d_out.alloc((size_t)nout * Jalloc * B));
+    B200SV_CUDA(d_mom.alloc(2));
+    B200SV_CUDA(d_sums.alloc(3 * (size_t)Jalloc));
+    return 0;
+  }
+
+  // payoffs of set b at maturity m (none without strikes) over the state (x, q) of n paths, re-centred with the moments in d_mom
+  int run(int b, int m, const void* x, const void* q, long long n, bool f32, double total_paths, cudaStream_t st) {
+    const int J = offsets[m + 1] - offsets[m], jo = offsets[m] - offsets[0];
+    if (J == 0) return 0;
+    const int kinds = payoff_kinds(types + offsets[m], J);
+    const int rc = f32 ? launch_payoff_t<float>(x, q, n, ttms[m], forwards[m], d_strikes.p + jo, d_types.p + jo, J, variable_type, kinds, d_mom.p, d_sums.p, st)
+                       : launch_payoff_t<double>(x, q, n, ttms[m], forwards[m], d_strikes.p + jo, d_types.p + jo, J, variable_type, kinds, d_mom.p, d_sums.p, st);
+    if (rc) return rc;
+    double* out = d_out.p + (size_t)nout * Jalloc * b;
+    const IvolSpec iv{d_strikes.p + jo, d_types.p + jo, forwards[m], ttms[m], nout == 3 ? out + 2 * Jalloc + jo : nullptr};
+    payoff_finalize_kernel<<<(J + 127) / 128, 128, 0, st>>>(d_sums.p, J, discfactors[m], total_paths, out + jo, out + Jalloc + jo, P2pGather{}, iv);
+    return launched("payoff_finalize_kernel");
+  }
+
+  // [B][Jtot] each; ivols only if the stage was made with them
+  int copy_back(double* prices, double* stderrs, double* ivols, cudaStream_t st) {
+    for (int b = 0; b < B && Jtot > 0; ++b) {
+      const double* out = d_out.p + (size_t)nout * Jalloc * b;
+      B200SV_CUDA(cudaMemcpyAsync(prices + (size_t)b * Jtot, out, sizeof(double) * Jtot, cudaMemcpyDeviceToHost, st));
+      B200SV_CUDA(cudaMemcpyAsync(stderrs + (size_t)b * Jtot, out + Jalloc, sizeof(double) * Jtot, cudaMemcpyDeviceToHost, st));
+      if (ivols) B200SV_CUDA(cudaMemcpyAsync(ivols + (size_t)b * Jtot, out + 2 * Jalloc, sizeof(double) * Jtot, cudaMemcpyDeviceToHost, st));
+    }
+    return 0;
+  }
+};
+
+// the SoA state [3][n] of a host-level call: three host arrays to and from one device buffer
+static int state_to_device(double* d, size_t n, const double* a, const double* b, const double* c, cudaStream_t st) {
+  B200SV_CUDA(cudaMemcpyAsync(d, a, sizeof(double) * n, cudaMemcpyHostToDevice, st));
+  B200SV_CUDA(cudaMemcpyAsync(d + n, b, sizeof(double) * n, cudaMemcpyHostToDevice, st));
+  B200SV_CUDA(cudaMemcpyAsync(d + 2 * n, c, sizeof(double) * n, cudaMemcpyHostToDevice, st));
+  return 0;
+}
+static int state_to_host(const double* d, size_t n, double* a, double* b, double* c, cudaStream_t st) {
+  B200SV_CUDA(cudaMemcpyAsync(a, d, sizeof(double) * n, cudaMemcpyDeviceToHost, st));
+  B200SV_CUDA(cudaMemcpyAsync(b, d + n, sizeof(double) * n, cudaMemcpyDeviceToHost, st));
+  B200SV_CUDA(cudaMemcpyAsync(c, d + 2 * n, sizeof(double) * n, cudaMemcpyDeviceToHost, st));
   return 0;
 }
 
+// the cooperative chain kernel of a model (fp64 state; kGaussF32 or kGaussF64 draws)
 template <int MODEL>
-static int coop_grid_blocks(int gauss, long long n) {
-  Grid g;
-  if (gauss == kGaussF64) {
-    if constexpr (MODEL == 0) g = persistent_grid(mc_chain_coop_kernel<LogsvPath<double>, LogsvConsts, kGaussF64>, kSliceThreads, n);
-    else if constexpr (MODEL == 1) g = persistent_grid(mc_chain_coop_kernel<HestonPath<double, false>, HestonConsts, kGaussF64>, kSliceThreads, n);
-    else g = persistent_grid(mc_chain_coop_kernel<HestonPath<double, true>, HestonConsts, kGaussF64>, kSliceThreads, n);
-  } else {
-    if constexpr (MODEL == 0) g = persistent_grid(mc_chain_coop_kernel<LogsvPath<double>, LogsvConsts, kGaussF32>, kSliceThreads, n);
-    else if constexpr (MODEL == 1) g = persistent_grid(mc_chain_coop_kernel<HestonPath<double, false>, HestonConsts, kGaussF32>, kSliceThreads, n);
-    else g = persistent_grid(mc_chain_coop_kernel<HestonPath<double, true>, HestonConsts, kGaussF32>, kSliceThreads, n);
-  }
-  return g.blocks;
-}
-
-template <int MODEL>
-static int launch_chain_coop(int gauss, const CoopArgs& args, const void* d_specs, int grid_blocks, cudaStream_t st) {
-  if (gauss == kGaussF64) return launch_chain_coop_g<MODEL, kGaussF64>(args, d_specs, grid_blocks, st);
-  return launch_chain_coop_g<MODEL, kGaussF32>(args, d_specs, grid_blocks, st);
+static const void* coop_kernel(int gauss) {
+  using CM = ChainModel<MODEL>;
+  if (gauss == kGaussF64) return (const void*)mc_chain_coop_kernel<typename CM::template Path<double>, typename CM::Consts, kGaussF64>;
+  return (const void*)mc_chain_coop_kernel<typename CM::template Path<double>, typename CM::Consts, kGaussF32>;
 }
 
 // Which chain driver?  The cooperative single-launch kernel wins where launch and host overhead matter (measured on B200, BTC chain,
@@ -1204,11 +1250,11 @@ static int mc_chain_host_coop(const b200sv_logsv_params* lp, const b200sv_heston
                               const double* discfactors, const double* etas, const int* offsets, const double* strikes, const int8_t* types,
                               long long nb_path, int nb_steps_per_year, int is_spot, int variable_type, uint64_t seed, int flags,
                               double* prices_out, double* stderr_out, int scheme, int B, double* ivols_out) {
-  using Spec = CoopSliceSpec<typename std::conditional<MODEL == 0, LogsvConsts, HestonConsts>::type>;
+  using Spec = CoopSliceSpec<typename ChainModel<MODEL>::Consts>;
   const int Jtot = offsets[M] - offsets[0], Jalloc = std::max(Jtot, 1);
   const int gauss = gauss_mode(flags);
-  const bool qe = MODEL == 1 && scheme == B200SV_HESTON_QE;
-  const int blocks = MODEL == 0 ? coop_grid_blocks<0>(gauss, nb_path) : (qe ? coop_grid_blocks<2>(gauss, nb_path) : coop_grid_blocks<1>(gauss, nb_path));
+  const void* kernel = MODEL == 0 ? coop_kernel<0>(gauss) : (scheme == B200SV_HESTON_QE ? coop_kernel<2>(gauss) : coop_kernel<1>(gauss));
+  const int blocks = persistent_grid(kernel, kSliceThreads, nb_path).blocks;
   int Jmax = 1;
   for (int m = 0; m < M; ++m) Jmax = std::max(Jmax, offsets[m + 1] - offsets[m]);
   const int Kpad_max = 3 * kStrikeChunk * ((Jmax + kStrikeChunk - 1) / kStrikeChunk);
@@ -1245,55 +1291,45 @@ static int mc_chain_host_coop(const b200sv_logsv_params* lp, const b200sv_heston
       sp.discfactor = discfactors[m];
     }
   }
-  cudaStream_t st = current_stream();
-  ensure_pool_threshold();
-  char* arena = nullptr;
-  B200SV_CUDA(cudaMallocAsync(&arena, total, st));
-  B200SV_CUDA(cudaMemcpyAsync(arena, h_in.data(), in_bytes, cudaMemcpyHostToDevice, st));      // pageable source: staged before the call returns
-  double* d_strikes = (double*)arena;
-  const Spec* d_specs = (const Spec*)(arena + sizeof(double) * Jalloc);
-  const int8_t* d_types = (const int8_t*)(arena + sizeof(double) * Jalloc + spec_bytes);
-  double* d_state = (double*)(arena + in_bytes);
-  double* d_out = d_state + 3 * (size_t)nb_path;
-  double* d_pm = d_out + out_doubles;
-  double* d_pp = d_pm + 2 * (size_t)blocks;
-  int rc = 0;
-  for (int b = 0; b < B && rc == 0; ++b) {
-    double* out_b = d_out + (size_t)3 * Jalloc * b;
-    CoopArgs a{};
-    a.x = d_state;
-    a.v = d_state + nb_path;
-    a.q = d_state + 2 * nb_path;
-    a.n = nb_path;
-    a.v_init = MODEL == 0 ? lp[b].sigma0 : hp[b].v0;
-    a.seed = seed;
-    a.M = M;
-    a.variable_type = variable_type;
-    a.strikes = d_strikes;
-    a.types = d_types;
-    a.part_mom = d_pm;
-    a.part_pay = d_pp;
-    a.Kpad_max = Kpad_max;
-    a.total_paths = (double)nb_path;
-    a.prices = out_b;
-    a.stderrs = out_b + Jalloc;
-    a.ivols = ivols_out ? out_b + 2 * Jalloc : nullptr;
-    const void* sp = d_specs + (size_t)b * M;
-    if (MODEL == 0)
-      rc = launch_chain_coop<0>(gauss, a, sp, blocks, st);
-    else if (qe)
-      rc = launch_chain_coop<2>(gauss, a, sp, blocks, st);
-    else
-      rc = launch_chain_coop<1>(gauss, a, sp, blocks, st);
-  }
   std::vector<double> h_out(out_doubles);
-  if (rc == 0 && Jtot > 0) {
-    cudaError_t e = cudaMemcpyAsync(h_out.data(), d_out, sizeof(double) * out_doubles, cudaMemcpyDeviceToHost, st);
-    if (e != cudaSuccess) rc = fail(-2, std::string("D2H: ") + cudaGetErrorString(e));
-  }
-  cudaFreeAsync(arena, st);
-  cudaError_t e = cudaStreamSynchronize(st);
-  if (rc == 0 && e != cudaSuccess) rc = fail(-2, std::string("sync: ") + cudaGetErrorString(e));
+  const int rc = host_call([&](cudaStream_t st) {
+    DevBuf<char> arena(st);
+    B200SV_CUDA(arena.alloc(total));
+    B200SV_CUDA(cudaMemcpyAsync(arena.p, h_in.data(), in_bytes, cudaMemcpyHostToDevice, st));      // pageable source: staged before the call returns
+    double* d_strikes = (double*)arena.p;
+    const Spec* d_specs = (const Spec*)(arena.p + sizeof(double) * Jalloc);
+    const int8_t* d_types = (const int8_t*)(arena.p + sizeof(double) * Jalloc + spec_bytes);
+    double* d_state = (double*)(arena.p + in_bytes);
+    double* d_out = d_state + 3 * (size_t)nb_path;
+    double* d_pm = d_out + out_doubles;
+    double* d_pp = d_pm + 2 * (size_t)blocks;
+    for (int b = 0; b < B; ++b) {
+      double* out_b = d_out + (size_t)3 * Jalloc * b;
+      CoopArgs a{};
+      a.x = d_state;
+      a.v = d_state + nb_path;
+      a.q = d_state + 2 * nb_path;
+      a.n = nb_path;
+      a.v_init = MODEL == 0 ? lp[b].sigma0 : hp[b].v0;
+      a.seed = seed;
+      a.M = M;
+      a.variable_type = variable_type;
+      a.strikes = d_strikes;
+      a.types = d_types;
+      a.part_mom = d_pm;
+      a.part_pay = d_pp;
+      a.Kpad_max = Kpad_max;
+      a.total_paths = (double)nb_path;
+      a.prices = out_b;
+      a.stderrs = out_b + Jalloc;
+      a.ivols = ivols_out ? out_b + 2 * Jalloc : nullptr;
+      const Spec* sp = d_specs + (size_t)b * M;
+      void* kargs[] = {(void*)&a, (void*)&sp};
+      if (int rc = launched("mc_chain_coop_kernel", cudaLaunchCooperativeKernel(kernel, dim3(blocks), dim3(kSliceThreads), kargs, 0, st))) return rc;
+    }
+    if (Jtot > 0) B200SV_CUDA(cudaMemcpyAsync(h_out.data(), d_out, sizeof(double) * out_doubles, cudaMemcpyDeviceToHost, st));
+    return 0;
+  });
   for (int b = 0; b < B && rc == 0 && Jtot > 0; ++b) {
     const double* o = h_out.data() + (size_t)3 * Jalloc * b;
     memcpy(prices_out + (size_t)b * Jtot, o, sizeof(double) * Jtot);
@@ -1319,71 +1355,35 @@ static int mc_chain_host(const b200sv_logsv_params* lp, const b200sv_heston_para
   if (use_coop_chain(flags, nb_path, MODEL == 1))
     return mc_chain_host_coop<MODEL>(lp, hp, M, ttms, forwards, discfactors, etas, offsets, strikes, types, nb_path, nb_steps_per_year, is_spot,
                                      variable_type, seed, flags, prices_out, stderr_out, scheme, B, ivols_out);
-  const int Jtot = offsets[M] - offsets[0];
-  const size_t esz = (flags & B200SV_STATE_F32) ? 4 : 8;
-  cudaStream_t st = current_stream();
-  ensure_pool_threshold();
-  char *x = nullptr;
-  double *d_strikes = nullptr, *d_out = nullptr, *d_mom = nullptr, *d_sums = nullptr;
-  int8_t* d_types = nullptr;
-  B200SV_CUDA(cudaMallocAsync(&x, 3 * esz * (size_t)nb_path, st));
-  char *v = x + esz * (size_t)nb_path, *q = x + 2 * esz * (size_t)nb_path;
-  const int Jalloc = std::max(Jtot, 1);
-  B200SV_CUDA(cudaMallocAsync(&d_strikes, sizeof(double) * Jalloc, st));
-  B200SV_CUDA(cudaMallocAsync(&d_types, Jalloc, st));
-  const size_t out_stride = (size_t)3 * Jalloc;                 // per set: prices, std errors, implied vols
-  B200SV_CUDA(cudaMallocAsync(&d_out, sizeof(double) * out_stride * B, st));
-  B200SV_CUDA(cudaMallocAsync(&d_mom, sizeof(double) * 2, st));
-  B200SV_CUDA(cudaMallocAsync(&d_sums, sizeof(double) * 3 * Jalloc, st));
-  if (Jtot > 0) {
-    B200SV_CUDA(cudaMemcpyAsync(d_strikes, strikes + offsets[0], sizeof(double) * Jtot, cudaMemcpyHostToDevice, st));
-    B200SV_CUDA(cudaMemcpyAsync(d_types, types + offsets[0], Jtot, cudaMemcpyHostToDevice, st));
-  }
-  int rc = 0;
-  for (int b = 0; b < B && rc == 0; ++b) {
-    double* out_b = d_out + out_stride * b;
-    double t0 = 0.0;
-    for (int m = 0; m < M && rc == 0; ++m) {
-      int S;
-      double dt;
-      time_grid(ttms[m] - t0, nb_steps_per_year, &S, &dt);
-      t0 = ttms[m];
-      if (MODEL == 0) {
-        const LogsvConsts c = make_logsv_consts(lp[b], etas ? etas[(size_t)b * M + m] : 1.0, is_spot != 0, dt);
-        rc = launch_slice<0>(x, v, q, nb_path, 0, m == 0, lp[b].sigma0, S, m, forwards[m], seed, flags, &c, nullptr, d_mom, st);
-      } else {
-        const HestonConsts c = make_heston_consts(hp[b], dt, scheme);
-        rc = launch_slice<1>(x, v, q, nb_path, 0, m == 0, hp[b].v0, S, m, forwards[m], seed, flags, nullptr, &c, d_mom, st);
+  if (int rc = check_slice_flags(flags)) return rc;
+  const bool f32 = flags & B200SV_STATE_F32;
+  const size_t esz = f32 ? 4 : 8;
+  return host_call([&](cudaStream_t st) {
+    DevBuf<char> x(st);
+    ChainPayoffs pay(st, M, ttms, forwards, discfactors, offsets, types, variable_type, B, ivols_out != nullptr);
+    B200SV_CUDA(x.alloc(3 * esz * (size_t)nb_path));
+    if (int rc = pay.alloc(strikes)) return rc;
+    char *v = x.p + esz * (size_t)nb_path, *q = x.p + 2 * esz * (size_t)nb_path;
+    for (int b = 0; b < B; ++b) {
+      double t0 = 0.0;
+      for (int m = 0; m < M; ++m) {
+        int S;
+        double dt;
+        time_grid(ttms[m] - t0, nb_steps_per_year, &S, &dt);
+        t0 = ttms[m];
+        int rc;
+        if constexpr (MODEL == 0)
+          rc = launch_slice<0>(x.p, v, q, nb_path, 0, m == 0, lp[b].sigma0, S, m, forwards[m], seed, flags,
+                               make_logsv_consts(lp[b], etas ? etas[(size_t)b * M + m] : 1.0, is_spot != 0, dt), pay.d_mom.p, st);
+        else
+          rc = launch_slice<1>(x.p, v, q, nb_path, 0, m == 0, hp[b].v0, S, m, forwards[m], seed, flags, make_heston_consts(hp[b], dt, scheme),
+                               pay.d_mom.p, st);
+        if (rc == 0) rc = pay.run(b, m, x.p, q, nb_path, f32, (double)nb_path, st);
+        if (rc) return rc;
       }
-      if (rc) break;
-      const int J = offsets[m + 1] - offsets[m], jo = offsets[m] - offsets[0];
-      if (J == 0) continue;
-      if (flags & B200SV_STATE_F32)
-        rc = launch_payoff_t<float>(x, q, nb_path, ttms[m], forwards[m], d_strikes + jo, d_types + jo, J, variable_type, payoff_kinds(types + offsets[m], J), d_mom, d_sums, st);
-      else
-        rc = launch_payoff_t<double>(x, q, nb_path, ttms[m], forwards[m], d_strikes + jo, d_types + jo, J, variable_type, payoff_kinds(types + offsets[m], J), d_mom, d_sums, st);
-      if (rc) break;
-      const IvolSpec iv{d_strikes + jo, d_types + jo, forwards[m], ttms[m], ivols_out ? out_b + 2 * Jalloc + jo : nullptr};
-      payoff_finalize_kernel<<<(J + 127) / 128, 128, 0, st>>>(d_sums, J, discfactors[m], (double)nb_path, out_b + jo, out_b + Jalloc + jo, P2pGather{}, iv);
-      rc = check_launch("payoff_finalize_kernel");
     }
-  }
-  for (int b = 0; b < B && rc == 0 && Jtot > 0; ++b) {
-    const double* out_b = d_out + out_stride * b;
-    cudaError_t e = cudaMemcpyAsync(prices_out + (size_t)b * Jtot, out_b, sizeof(double) * Jtot, cudaMemcpyDeviceToHost, st);
-    if (e == cudaSuccess) e = cudaMemcpyAsync(stderr_out + (size_t)b * Jtot, out_b + Jalloc, sizeof(double) * Jtot, cudaMemcpyDeviceToHost, st);
-    if (e == cudaSuccess && ivols_out) e = cudaMemcpyAsync(ivols_out + (size_t)b * Jtot, out_b + 2 * Jalloc, sizeof(double) * Jtot, cudaMemcpyDeviceToHost, st);
-    if (e != cudaSuccess) rc = fail(-2, std::string("D2H: ") + cudaGetErrorString(e));
-  }
-  cudaFreeAsync(x, st);
-  cudaFreeAsync(d_strikes, st);
-  cudaFreeAsync(d_types, st);
-  cudaFreeAsync(d_out, st);
-  cudaFreeAsync(d_mom, st);
-  cudaFreeAsync(d_sums, st);
-  cudaError_t e = cudaStreamSynchronize(st);
-  if (rc == 0 && e != cudaSuccess) rc = fail(-2, std::string("sync: ") + cudaGetErrorString(e));
-  return rc;
+    return pay.copy_back(prices_out, stderr_out, ivols_out, st);
+  });
 }
 
 template <int MODEL>
@@ -1391,33 +1391,23 @@ static int terminal_host(const b200sv_logsv_params* lp, const b200sv_heston_para
                          int nb_steps_per_year, int is_spot, double eta, uint64_t seed, int flags, double* x, double* v, double* q, int scheme = 0) {
   B200SV_REQUIRE(nb_path >= 1 && ttm > 0.0 && nb_steps_per_year >= 1, "nb_path, ttm, nb_steps_per_year must be positive");
   B200SV_REQUIRE(!(flags & B200SV_STATE_F32), "terminal values are returned as float64: use B200SV_STATE_F64");
-  cudaStream_t st = current_stream();
-  ensure_pool_threshold();
-  double *d = nullptr, *d_mom = nullptr;
-  B200SV_CUDA(cudaMallocAsync(&d, sizeof(double) * 3 * (size_t)nb_path, st));
-  B200SV_CUDA(cudaMallocAsync(&d_mom, sizeof(double) * 2, st));
+  if (int rc = check_slice_flags(flags)) return rc;
   int S;
   double dt;
   time_grid(ttm, nb_steps_per_year, &S, &dt);
-  int rc;
-  if (MODEL == 0) {
-    const LogsvConsts c = make_logsv_consts(*lp, eta, is_spot != 0, dt);
-    rc = launch_slice<0>(d, d + nb_path, d + 2 * nb_path, nb_path, 0, 1, lp->sigma0, S, 0, 1.0, seed, flags, &c, nullptr, d_mom, st);
-  } else {
-    const HestonConsts c = make_heston_consts(*hp, dt, scheme);
-    rc = launch_slice<1>(d, d + nb_path, d + 2 * nb_path, nb_path, 0, 1, hp->v0, S, 0, 1.0, seed, flags, nullptr, &c, d_mom, st);
-  }
-  if (rc == 0) {
-    cudaError_t e = cudaMemcpyAsync(x, d, sizeof(double) * nb_path, cudaMemcpyDeviceToHost, st);
-    if (e == cudaSuccess) e = cudaMemcpyAsync(v, d + nb_path, sizeof(double) * nb_path, cudaMemcpyDeviceToHost, st);
-    if (e == cudaSuccess) e = cudaMemcpyAsync(q, d + 2 * nb_path, sizeof(double) * nb_path, cudaMemcpyDeviceToHost, st);
-    if (e != cudaSuccess) rc = fail(-2, std::string("D2H: ") + cudaGetErrorString(e));
-  }
-  cudaFreeAsync(d, st);
-  cudaFreeAsync(d_mom, st);
-  cudaError_t e = cudaStreamSynchronize(st);
-  if (rc == 0 && e != cudaSuccess) rc = fail(-2, std::string("sync: ") + cudaGetErrorString(e));
-  return rc;
+  return host_call([&](cudaStream_t st) {
+    DevBuf<double> d(st), d_mom(st);
+    B200SV_CUDA(d.alloc(3 * (size_t)nb_path));
+    B200SV_CUDA(d_mom.alloc(2));
+    int rc;
+    if constexpr (MODEL == 0)
+      rc = launch_slice<0>(d.p, d.p + nb_path, d.p + 2 * nb_path, nb_path, 0, 1, lp->sigma0, S, 0, 1.0, seed, flags,
+                           make_logsv_consts(*lp, eta, is_spot != 0, dt), d_mom.p, st);
+    else
+      rc = launch_slice<1>(d.p, d.p + nb_path, d.p + 2 * nb_path, nb_path, 0, 1, hp->v0, S, 0, 1.0, seed, flags, make_heston_consts(*hp, dt, scheme),
+                           d_mom.p, st);
+    return rc ? rc : state_to_host(d.p, nb_path, x, v, q, st);
+  });
 }
 
 }  // namespace b200sv
@@ -1437,11 +1427,8 @@ int b200sv_set_stream(void* stream) {
   return 0;
 }
 void* b200sv_get_stream(void) { return (void*)current_stream(); }
-long long b200sv_launch_count(void) { return g_launches; }
-void b200sv_reset_launch_count(void) { g_launches = 0; }
-
-// internal hook for the MGF translation unit
-void b200sv_internal_count_launch(void) { ++g_launches; }
+long long b200sv_launch_count(void) { return launch_count(); }
+void b200sv_reset_launch_count(void) { launch_count() = 0; }
 
 int b200sv_logsv_mc_chain(const b200sv_logsv_params* params, int M, const double* ttms, const double* forwards,
                           const double* discfactors, const double* etas, const int* offsets, const double* strikes,
@@ -1496,31 +1483,20 @@ int b200sv_logsv_terminal_from_state(const b200sv_logsv_params* params, double t
   B200SV_REQUIRE(params && x_inout && sigma_inout && qvar_inout, "null pointer");
   B200SV_REQUIRE(nb_path >= 1 && ttm > 0.0 && nb_steps_per_year >= 1 && slice_index >= 0, "nb_path, ttm, nb_steps_per_year must be positive");
   B200SV_REQUIRE(!(flags & B200SV_STATE_F32), "terminal values are returned as float64: use B200SV_STATE_F64");
-  cudaStream_t st = current_stream();
-  ensure_pool_threshold();
-  double *d = nullptr, *d_mom = nullptr;
-  const size_t nb = sizeof(double) * (size_t)nb_path;
-  B200SV_CUDA(cudaMallocAsync(&d, 3 * nb, st));
-  B200SV_CUDA(cudaMallocAsync(&d_mom, sizeof(double) * 2, st));
-  B200SV_CUDA(cudaMemcpyAsync(d, x_inout, nb, cudaMemcpyHostToDevice, st));
-  B200SV_CUDA(cudaMemcpyAsync(d + nb_path, sigma_inout, nb, cudaMemcpyHostToDevice, st));
-  B200SV_CUDA(cudaMemcpyAsync(d + 2 * nb_path, qvar_inout, nb, cudaMemcpyHostToDevice, st));
+  if (int rc = check_slice_flags(flags)) return rc;
   int S;
   double dt;
   time_grid(ttm, nb_steps_per_year, &S, &dt);
   const LogsvConsts c = make_logsv_consts(*params, eta, is_spot_measure != 0, dt);
-  int rc = launch_slice<0>(d, d + nb_path, d + 2 * nb_path, nb_path, 0, 0, params->sigma0, S, slice_index, 1.0, seed, flags, &c, nullptr, d_mom, st);
-  if (rc == 0) {
-    cudaError_t e = cudaMemcpyAsync(x_inout, d, nb, cudaMemcpyDeviceToHost, st);
-    if (e == cudaSuccess) e = cudaMemcpyAsync(sigma_inout, d + nb_path, nb, cudaMemcpyDeviceToHost, st);
-    if (e == cudaSuccess) e = cudaMemcpyAsync(qvar_inout, d + 2 * nb_path, nb, cudaMemcpyDeviceToHost, st);
-    if (e != cudaSuccess) rc = fail(-2, std::string("D2H: ") + cudaGetErrorString(e));
-  }
-  cudaFreeAsync(d, st);
-  cudaFreeAsync(d_mom, st);
-  cudaError_t e = cudaStreamSynchronize(st);
-  if (rc == 0 && e != cudaSuccess) rc = fail(-2, std::string("sync: ") + cudaGetErrorString(e));
-  return rc;
+  return host_call([&](cudaStream_t st) {
+    DevBuf<double> d(st), d_mom(st);
+    B200SV_CUDA(d.alloc(3 * (size_t)nb_path));
+    B200SV_CUDA(d_mom.alloc(2));
+    if (int rc = state_to_device(d.p, nb_path, x_inout, sigma_inout, qvar_inout, st)) return rc;
+    if (int rc = launch_slice<0>(d.p, d.p + nb_path, d.p + 2 * nb_path, nb_path, 0, 0, params->sigma0, S, slice_index, 1.0, seed, flags, c, d_mom.p, st))
+      return rc;
+    return state_to_host(d.p, nb_path, x_inout, sigma_inout, qvar_inout, st);
+  });
 }
 
 int b200sv_heston_terminal(const b200sv_heston_params* params, double ttm, long long nb_path, int nb_steps_per_year,
@@ -1537,8 +1513,8 @@ int b200sv_dev_logsv_slice(void* x, void* sigma, void* qvar, long long n_local, 
   B200SV_REQUIRE(x && sigma && qvar && params && moments_out, "null pointer");
   B200SV_REQUIRE(n_local >= 1 && nsteps >= 1 && dt > 0.0, "n_local, nsteps, dt must be positive");
   const LogsvConsts c = make_logsv_consts(*params, eta, is_spot_measure != 0, dt);
-  return launch_slice<0>(x, sigma, qvar, n_local, path_offset, init, params->sigma0, nsteps, slice_index, forward, seed, flags,
-                         &c, nullptr, moments_out, (cudaStream_t)stream, (P2pCtx*)p2p);
+  return launch_slice<0>(x, sigma, qvar, n_local, path_offset, init, params->sigma0, nsteps, slice_index, forward, seed, flags, c,
+                         moments_out, (cudaStream_t)stream, (P2pCtx*)p2p);
 }
 
 int b200sv_dev_heston_slice(void* x, void* var, void* qvar, long long n_local, long long path_offset, int init,
@@ -1548,8 +1524,8 @@ int b200sv_dev_heston_slice(void* x, void* var, void* qvar, long long n_local, l
   B200SV_REQUIRE(n_local >= 1 && nsteps >= 1 && dt > 0.0, "n_local, nsteps, dt must be positive");
   B200SV_REQUIRE(scheme == B200SV_HESTON_EULER_FLOOR || scheme == B200SV_HESTON_QE, "unknown Heston scheme");
   const HestonConsts c = make_heston_consts(*params, dt, scheme);
-  return launch_slice<1>(x, var, qvar, n_local, path_offset, init, params->v0, nsteps, slice_index, forward, seed, flags, nullptr,
-                         &c, moments_out, (cudaStream_t)stream, (P2pCtx*)p2p);
+  return launch_slice<1>(x, var, qvar, n_local, path_offset, init, params->v0, nsteps, slice_index, forward, seed, flags, c,
+                         moments_out, (cudaStream_t)stream, (P2pCtx*)p2p);
 }
 
 int b200sv_dev_payoff_sums(const void* x, const void* qvar, long long n_local, int flags, double ttm, double forward,
@@ -1570,7 +1546,7 @@ int b200sv_dev_payoff_finalize(const double* sums, int J, double discfactor, lon
   // exchange #2 (consumer): with a P2P context the global sums are gathered from the mailbox, `sums` holds this rank's local ones
   payoff_finalize_kernel<<<(J + 127) / 128, 128, 0, (cudaStream_t)stream>>>(sums, J, discfactor, (double)total_paths, prices_out, stderr_out,
                                                                             make_gather((P2pCtx*)p2p));
-  return check_launch("payoff_finalize_kernel");
+  return launched("payoff_finalize_kernel");
 }
 
 int b200sv_dev_logsv_step_fixed(double* x, double* sigma, double* qvar, const double* W0, const double* W1, int S, long long N,
@@ -1581,13 +1557,13 @@ int b200sv_dev_logsv_step_fixed(double* x, double* sigma, double* qvar, const do
     const LogsvConsts c = make_logsv_consts(*params, eta, is_spot_measure != 0, dt);
     Grid g = persistent_grid(logsv_step_fixed_fast_kernel, kThreads, N);
     logsv_step_fixed_fast_kernel<<<g.blocks, g.threads, 0, (cudaStream_t)stream>>>(x, sigma, qvar, W0, W1, S, N, c);
-    return check_launch("logsv_step_fixed_fast_kernel");
+    return launched("logsv_step_fixed_fast_kernel");
   }
   LogsvRaw r{params->theta, params->kappa1, params->kappa2, params->beta, params->volvol, eta,
              is_spot_measure ? -1.0 : 1.0, is_spot_measure ? 0.0 : params->beta * eta, dt};
   Grid g = persistent_grid(logsv_step_fixed_kernel, kThreads, N);
   logsv_step_fixed_kernel<<<g.blocks, g.threads, 0, (cudaStream_t)stream>>>(x, sigma, qvar, W0, W1, S, N, r);
-  return check_launch("logsv_step_fixed_kernel");
+  return launched("logsv_step_fixed_kernel");
 }
 
 int b200sv_dev_heston_step_fixed(double* x, double* var, double* qvar, const double* W0, const double* W1, int S, long long N,
@@ -1596,20 +1572,18 @@ int b200sv_dev_heston_step_fixed(double* x, double* var, double* qvar, const dou
   B200SV_REQUIRE(S >= 0 && N >= 1 && dt > 0.0, "S, N, dt");
   Grid g = persistent_grid(heston_step_fixed_kernel, kThreads, N);
   heston_step_fixed_kernel<<<g.blocks, g.threads, 0, (cudaStream_t)stream>>>(x, var, qvar, W0, W1, S, N, *params, dt);
-  return check_launch("heston_step_fixed_kernel");
+  return launched("heston_step_fixed_kernel");
 }
 
 static int spot_moments_impl(const double* x, long long n, double forward, double* moments_out, cudaStream_t st, P2pCtx* p2p) {
   Grid g = persistent_grid(spot_moments_kernel, kThreads, n);
-  double* partials = nullptr;
+  DevBuf<double> partials(st);
   ensure_pool_threshold();
-  B200SV_CUDA(cudaMallocAsync(&partials, sizeof(double) * 2 * g.blocks, st));
-  spot_moments_kernel<<<g.blocks, g.threads, 0, st>>>(x, n, forward, partials);
-  if (int rc = check_launch("spot_moments_kernel")) return rc;
-  reduce_partials_kernel<<<1, 64, 0, st>>>(partials, g.blocks, 2, 2, moments_out, make_publish(p2p, st));
-  if (int rc = check_launch("reduce_partials_kernel")) return rc;
-  B200SV_CUDA(cudaFreeAsync(partials, st));
-  return 0;
+  B200SV_CUDA(partials.alloc(2 * (size_t)g.blocks));
+  spot_moments_kernel<<<g.blocks, g.threads, 0, st>>>(x, n, forward, partials.p);
+  if (int rc = launched("spot_moments_kernel")) return rc;
+  reduce_partials_kernel<<<1, 64, 0, st>>>(partials.p, g.blocks, 2, 2, moments_out, make_publish(p2p, st));
+  return launched("reduce_partials_kernel");
 }
 
 int b200sv_dev_spot_moments(const double* x, long long n, double forward, double* moments_out, void* stream) {
@@ -1650,31 +1624,20 @@ static int step_fixed_host(int model, double* x, double* v, double* q, const dou
                            double dt, const b200sv_logsv_params* lp, double eta, int is_spot, const b200sv_heston_params* hp) {
   B200SV_REQUIRE(x && v && q && (S == 0 || (W0 && W1)), "null pointer");
   B200SV_REQUIRE(S >= 0 && N >= 1 && dt > 0.0, "S, N, dt");
-  cudaStream_t st = current_stream();
-  double *d = nullptr, *w = nullptr;
-  const size_t nb = sizeof(double) * (size_t)N, wb = sizeof(double) * (size_t)N * (size_t)std::max(S, 1);
-  B200SV_CUDA(cudaMallocAsync(&d, 3 * nb, st));
-  B200SV_CUDA(cudaMallocAsync(&w, 2 * wb, st));
-  B200SV_CUDA(cudaMemcpyAsync(d, x, nb, cudaMemcpyHostToDevice, st));
-  B200SV_CUDA(cudaMemcpyAsync(d + N, v, nb, cudaMemcpyHostToDevice, st));
-  B200SV_CUDA(cudaMemcpyAsync(d + 2 * N, q, nb, cudaMemcpyHostToDevice, st));
-  if (S > 0) {
-    B200SV_CUDA(cudaMemcpyAsync(w, W0, wb, cudaMemcpyHostToDevice, st));
-    B200SV_CUDA(cudaMemcpyAsync(w + (size_t)N * S, W1, wb, cudaMemcpyHostToDevice, st));
-  }
-  int rc = model == 0 ? b200sv_dev_logsv_step_fixed(d, d + N, d + 2 * N, w, w + (size_t)N * S, S, N, dt, lp, eta, is_spot, 0, st)
-                      : b200sv_dev_heston_step_fixed(d, d + N, d + 2 * N, w, w + (size_t)N * S, S, N, dt, hp, st);
-  if (rc == 0) {
-    cudaError_t e = cudaMemcpyAsync(x, d, nb, cudaMemcpyDeviceToHost, st);
-    if (e == cudaSuccess) e = cudaMemcpyAsync(v, d + N, nb, cudaMemcpyDeviceToHost, st);
-    if (e == cudaSuccess) e = cudaMemcpyAsync(q, d + 2 * N, nb, cudaMemcpyDeviceToHost, st);
-    if (e != cudaSuccess) rc = fail(-2, std::string("D2H: ") + cudaGetErrorString(e));
-  }
-  cudaFreeAsync(d, st);
-  cudaFreeAsync(w, st);
-  cudaError_t e = cudaStreamSynchronize(st);
-  if (rc == 0 && e != cudaSuccess) rc = fail(-2, std::string("sync: ") + cudaGetErrorString(e));
-  return rc;
+  const size_t wn = (size_t)N * S;
+  return host_call([&](cudaStream_t st) {
+    DevBuf<double> d(st), w(st);
+    B200SV_CUDA(d.alloc(3 * (size_t)N));
+    B200SV_CUDA(w.alloc(2 * std::max<size_t>(wn, N)));
+    if (int rc = state_to_device(d.p, N, x, v, q, st)) return rc;
+    if (S > 0) {
+      B200SV_CUDA(cudaMemcpyAsync(w.p, W0, sizeof(double) * wn, cudaMemcpyHostToDevice, st));
+      B200SV_CUDA(cudaMemcpyAsync(w.p + wn, W1, sizeof(double) * wn, cudaMemcpyHostToDevice, st));
+    }
+    const int rc = model == 0 ? b200sv_dev_logsv_step_fixed(d.p, d.p + N, d.p + 2 * N, w.p, w.p + wn, S, N, dt, lp, eta, is_spot, 0, st)
+                              : b200sv_dev_heston_step_fixed(d.p, d.p + N, d.p + 2 * N, w.p, w.p + wn, S, N, dt, hp, st);
+    return rc ? rc : state_to_host(d.p, N, x, v, q, st);
+  });
 }
 
 int b200sv_logsv_step_fixed(double* x, double* sigma, double* qvar, const double* W0, const double* W1, int S, long long N,
@@ -1697,96 +1660,66 @@ int b200sv_mc_payoffs(const double* x, const double* qvar, long long N, double t
     if (types[j] < 0 || types[j] > 3) return fail(-3, "unknown option payoff code");
   if (variable_type != B200SV_LOG_RETURN && variable_type != B200SV_Q_VAR) return fail(-4, "variable_type not implemented");
   B200SV_REQUIRE(variable_type == B200SV_LOG_RETURN || qvar, "qvar required for Q_VAR");
-  cudaStream_t st = current_stream();
-  double *d = nullptr, *dk = nullptr, *d_mom = nullptr, *d_sums = nullptr, *d_out = nullptr;
-  int8_t* dt_ = nullptr;
-  const size_t nb = sizeof(double) * (size_t)N;
-  B200SV_CUDA(cudaMallocAsync(&d, 2 * nb, st));
-  B200SV_CUDA(cudaMallocAsync(&dk, sizeof(double) * J, st));
-  B200SV_CUDA(cudaMallocAsync(&dt_, J, st));
-  B200SV_CUDA(cudaMallocAsync(&d_mom, sizeof(double) * 2, st));
-  B200SV_CUDA(cudaMallocAsync(&d_sums, sizeof(double) * 3 * J, st));
-  B200SV_CUDA(cudaMallocAsync(&d_out, sizeof(double) * 2 * J, st));
-  B200SV_CUDA(cudaMemcpyAsync(d, x, nb, cudaMemcpyHostToDevice, st));
-  if (qvar) B200SV_CUDA(cudaMemcpyAsync(d + N, qvar, nb, cudaMemcpyHostToDevice, st));
-  B200SV_CUDA(cudaMemcpyAsync(dk, strikes, sizeof(double) * J, cudaMemcpyHostToDevice, st));
-  B200SV_CUDA(cudaMemcpyAsync(dt_, types, J, cudaMemcpyHostToDevice, st));
-  int rc = b200sv_dev_spot_moments(d, N, forward, d_mom, st);
-  if (rc == 0) rc = launch_payoff_t<double>(d, d + N, N, ttm, forward, dk, dt_, J, variable_type, payoff_kinds(types, J), d_mom, d_sums, st);
-  if (rc == 0) rc = b200sv_dev_payoff_finalize(d_sums, J, discfactor, N, d_out, d_out + J, nullptr, st);
-  if (rc == 0) {
-    cudaError_t e = cudaMemcpyAsync(prices_out, d_out, sizeof(double) * J, cudaMemcpyDeviceToHost, st);
-    if (e == cudaSuccess) e = cudaMemcpyAsync(stderr_out, d_out + J, sizeof(double) * J, cudaMemcpyDeviceToHost, st);
-    if (e != cudaSuccess) rc = fail(-2, std::string("D2H: ") + cudaGetErrorString(e));
-  }
-  cudaFreeAsync(d, st);
-  cudaFreeAsync(dk, st);
-  cudaFreeAsync(dt_, st);
-  cudaFreeAsync(d_mom, st);
-  cudaFreeAsync(d_sums, st);
-  cudaFreeAsync(d_out, st);
-  cudaError_t e = cudaStreamSynchronize(st);
-  if (rc == 0 && e != cudaSuccess) rc = fail(-2, std::string("sync: ") + cudaGetErrorString(e));
-  return rc;
+  const int offsets[2] = {0, J};
+  return host_call([&](cudaStream_t st) {
+    DevBuf<double> d(st);
+    ChainPayoffs pay(st, 1, &ttm, &forward, &discfactor, offsets, types, variable_type, 1, false);
+    B200SV_CUDA(d.alloc(2 * (size_t)N));
+    if (int rc = pay.alloc(strikes)) return rc;
+    B200SV_CUDA(cudaMemcpyAsync(d.p, x, sizeof(double) * N, cudaMemcpyHostToDevice, st));
+    if (qvar) B200SV_CUDA(cudaMemcpyAsync(d.p + N, qvar, sizeof(double) * N, cudaMemcpyHostToDevice, st));
+    if (int rc = spot_moments_impl(d.p, N, forward, pay.d_mom.p, st, nullptr)) return rc;
+    if (int rc = pay.run(0, 0, d.p, d.p + N, N, false, (double)N, st)) return rc;
+    return pay.copy_back(prices_out, stderr_out, nullptr, st);
+  });
 }
 
 int b200sv_device_normals(uint64_t seed, long long path0, long long n, int slice, int nsteps, int flags, double* z0, double* z1) {
   B200SV_REQUIRE(z0 && z1 && n >= 1 && nsteps >= 1, "null pointer / sizes");
-  cudaStream_t st = current_stream();
-  double* d = nullptr;
-  const size_t nb = sizeof(double) * (size_t)n * nsteps;
-  B200SV_CUDA(cudaMallocAsync(&d, 2 * nb, st));
-  const int blocks = (int)((n + 127) / 128);
   const int g = gauss_mode(flags);
   B200SV_REQUIRE(g >= 0, "B200SV_GAUSS_F64 and B200SV_GAUSS_F64_PAIRED are mutually exclusive");
-  if (g == kGaussF64)
-    device_normals_kernel<kGaussF64><<<blocks, 128, 0, st>>>(seed, (unsigned long long)path0, n, (unsigned)slice, nsteps, d, d + (size_t)n * nsteps);
-  else if (g == kGaussF64Paired)
-    device_normals_kernel<kGaussF64Paired><<<blocks, 128, 0, st>>>(seed, (unsigned long long)path0, n, (unsigned)slice, nsteps, d, d + (size_t)n * nsteps);
-  else
-    device_normals_kernel<kGaussF32><<<blocks, 128, 0, st>>>(seed, (unsigned long long)path0, n, (unsigned)slice, nsteps, d, d + (size_t)n * nsteps);
-  int rc = check_launch("device_normals_kernel");
-  if (rc == 0) {
-    cudaError_t e = cudaMemcpyAsync(z0, d, nb, cudaMemcpyDeviceToHost, st);
-    if (e == cudaSuccess) e = cudaMemcpyAsync(z1, d + (size_t)n * nsteps, nb, cudaMemcpyDeviceToHost, st);
-    if (e != cudaSuccess) rc = fail(-2, std::string("D2H: ") + cudaGetErrorString(e));
-  }
-  cudaFreeAsync(d, st);
-  cudaError_t e = cudaStreamSynchronize(st);
-  if (rc == 0 && e != cudaSuccess) rc = fail(-2, std::string("sync: ") + cudaGetErrorString(e));
-  return rc;
+  const size_t nz = (size_t)n * nsteps;
+  return host_call([&](cudaStream_t st) {
+    DevBuf<double> d(st);
+    B200SV_CUDA(d.alloc(2 * nz));
+    const int blocks = (int)((n + 127) / 128);
+    if (g == kGaussF64)
+      device_normals_kernel<kGaussF64><<<blocks, 128, 0, st>>>(seed, (unsigned long long)path0, n, (unsigned)slice, nsteps, d.p, d.p + nz);
+    else if (g == kGaussF64Paired)
+      device_normals_kernel<kGaussF64Paired><<<blocks, 128, 0, st>>>(seed, (unsigned long long)path0, n, (unsigned)slice, nsteps, d.p, d.p + nz);
+    else
+      device_normals_kernel<kGaussF32><<<blocks, 128, 0, st>>>(seed, (unsigned long long)path0, n, (unsigned)slice, nsteps, d.p, d.p + nz);
+    if (int rc = launched("device_normals_kernel")) return rc;
+    B200SV_CUDA(cudaMemcpyAsync(z0, d.p, sizeof(double) * nz, cudaMemcpyDeviceToHost, st));
+    B200SV_CUDA(cudaMemcpyAsync(z1, d.p + nz, sizeof(double) * nz, cudaMemcpyDeviceToHost, st));
+    return 0;
+  });
 }
 
 int b200sv_debug_exp_pair_scaled(const double* Ls, long long n, double* out /* 2n */) {
   B200SV_REQUIRE(Ls && out && n >= 1, "null pointer / n");
-  cudaStream_t st = current_stream();
-  double *dl = nullptr, *dout = nullptr;
-  B200SV_CUDA(cudaMallocAsync(&dl, sizeof(double) * n, st));
-  B200SV_CUDA(cudaMallocAsync(&dout, sizeof(double) * 2 * n, st));
-  B200SV_CUDA(cudaMemcpyAsync(dl, Ls, sizeof(double) * n, cudaMemcpyHostToDevice, st));
-  exp_pair_scaled_kernel<<<(int)((n + 127) / 128), 128, 0, st>>>(dl, n, dout);
-  int rc = check_launch("exp_pair_scaled_kernel");
-  if (rc == 0) B200SV_CUDA(cudaMemcpyAsync(out, dout, sizeof(double) * 2 * n, cudaMemcpyDeviceToHost, st));
-  cudaFreeAsync(dl, st);
-  cudaFreeAsync(dout, st);
-  B200SV_CUDA(cudaStreamSynchronize(st));
-  return rc;
+  return host_call([&](cudaStream_t st) {
+    DevBuf<double> dl(st), dout(st);
+    B200SV_CUDA(dl.upload(Ls, n));
+    B200SV_CUDA(dout.alloc(2 * (size_t)n));
+    exp_pair_scaled_kernel<<<(int)((n + 127) / 128), 128, 0, st>>>(dl.p, n, dout.p);
+    if (int rc = launched("exp_pair_scaled_kernel")) return rc;
+    B200SV_CUDA(cudaMemcpyAsync(out, dout.p, sizeof(double) * 2 * n, cudaMemcpyDeviceToHost, st));
+    return 0;
+  });
 }
 
 int b200sv_debug_exp_pair(const double* L, long long n, double* out /* 2n */) {
   B200SV_REQUIRE(L && out && n >= 1, "null pointer / n");
-  cudaStream_t st = current_stream();
-  double *dl = nullptr, *dout = nullptr;
-  B200SV_CUDA(cudaMallocAsync(&dl, sizeof(double) * n, st));
-  B200SV_CUDA(cudaMallocAsync(&dout, sizeof(double) * 2 * n, st));
-  B200SV_CUDA(cudaMemcpyAsync(dl, L, sizeof(double) * n, cudaMemcpyHostToDevice, st));
-  exp_pair_kernel<<<(int)((n + 127) / 128), 128, 0, st>>>(dl, n, dout);
-  int rc = check_launch("exp_pair_kernel");
-  if (rc == 0) B200SV_CUDA(cudaMemcpyAsync(out, dout, sizeof(double) * 2 * n, cudaMemcpyDeviceToHost, st));
-  cudaFreeAsync(dl, st);
-  cudaFreeAsync(dout, st);
-  B200SV_CUDA(cudaStreamSynchronize(st));
-  return rc;
+  return host_call([&](cudaStream_t st) {
+    DevBuf<double> dl(st), dout(st);
+    B200SV_CUDA(dl.upload(L, n));
+    B200SV_CUDA(dout.alloc(2 * (size_t)n));
+    exp_pair_kernel<<<(int)((n + 127) / 128), 128, 0, st>>>(dl.p, n, dout.p);
+    if (int rc = launched("exp_pair_kernel")) return rc;
+    B200SV_CUDA(cudaMemcpyAsync(out, dout.p, sizeof(double) * 2 * n, cudaMemcpyDeviceToHost, st));
+    return 0;
+  });
 }
 
 int b200sv_logsv_vol_paths(const b200sv_logsv_params* params, double ttm, long long nb_path, int nb_steps_per_year, int is_spot_measure,
@@ -1799,27 +1732,17 @@ int b200sv_logsv_vol_paths(const b200sv_logsv_params* params, double ttm, long l
   // adj = beta under the inverse measure, no eta (pricers/logsv_pricer.py:929-932)
   LogsvRaw r{params->theta, params->kappa1, params->kappa2, params->beta, params->volvol, 1.0, is_spot_measure ? -1.0 : 1.0,
              is_spot_measure ? 0.0 : params->beta, dt};
-  cudaStream_t st = current_stream();
-  ensure_pool_threshold();
-  double *d_out = nullptr, *d_w = nullptr;
-  const size_t ob = sizeof(double) * (size_t)(S + 1) * (size_t)nb_path, wb = sizeof(double) * (size_t)S * (size_t)nb_path;
-  B200SV_CUDA(cudaMallocAsync(&d_out, ob, st));
-  if (brownians) {
-    B200SV_CUDA(cudaMallocAsync(&d_w, wb, st));
-    B200SV_CUDA(cudaMemcpyAsync(d_w, brownians, wb, cudaMemcpyHostToDevice, st));
-  }
-  Grid g = persistent_grid(logsv_vol_paths_kernel, kThreads, nb_path);
-  logsv_vol_paths_kernel<<<g.blocks, g.threads, 0, st>>>(d_out, d_w, S, nb_path, r, params->sigma0, seed, 0ull);
-  int rc = check_launch("logsv_vol_paths_kernel");
-  if (rc == 0) {
-    cudaError_t e = cudaMemcpyAsync(sigma_t_out, d_out, ob, cudaMemcpyDeviceToHost, st);
-    if (e != cudaSuccess) rc = fail(-2, std::string("D2H: ") + cudaGetErrorString(e));
-  }
-  cudaFreeAsync(d_out, st);
-  if (d_w) cudaFreeAsync(d_w, st);
-  cudaError_t e = cudaStreamSynchronize(st);
-  if (rc == 0 && e != cudaSuccess) rc = fail(-2, std::string("sync: ") + cudaGetErrorString(e));
-  return rc;
+  const size_t ob = (size_t)(S + 1) * (size_t)nb_path;
+  return host_call([&](cudaStream_t st) {
+    DevBuf<double> d_out(st), d_w(st);
+    B200SV_CUDA(d_out.alloc(ob));
+    if (brownians) B200SV_CUDA(d_w.upload(brownians, (size_t)S * (size_t)nb_path));
+    Grid g = persistent_grid(logsv_vol_paths_kernel, kThreads, nb_path);
+    logsv_vol_paths_kernel<<<g.blocks, g.threads, 0, st>>>(d_out.p, d_w.p, S, nb_path, r, params->sigma0, seed, 0ull);
+    if (int rc = launched("logsv_vol_paths_kernel")) return rc;
+    B200SV_CUDA(cudaMemcpyAsync(sigma_t_out, d_out.p, sizeof(double) * ob, cudaMemcpyDeviceToHost, st));
+    return 0;
+  });
 }
 
 // ---- rough-LogSV multi-factor MC (rough_kernels.cuh) ------------------------------------------------------------------------
@@ -1839,73 +1762,49 @@ int b200sv_hawkesjd_mc_chain(const b200sv_hawkes_params* params, int M, const do
                              int flags, double* prices_out, double* stderr_out) {
   B200SV_REQUIRE(params && ttms && forwards && discfactors && offsets && prices_out && stderr_out, "null pointer");
   return hawkes_chain_host(params, M, ttms, forwards, discfactors, offsets, strikes, types, nb_path, variable_type, seed, flags, prices_out,
-                           stderr_out, nullptr);
+                           stderr_out);
 }
 
 int b200sv_hawkesjd_terminal(const b200sv_hawkes_params* params, double ttm, long long nb_path, uint64_t seed, int flags, int slice_index,
                              int use_initial_arrays, double* x_inout, double* lambda_p_inout, double* lambda_m_inout) {
   B200SV_REQUIRE(params && x_inout && lambda_p_inout && lambda_m_inout, "null pointer");
   B200SV_REQUIRE(nb_path >= 1 && ttm > 0.0 && slice_index >= 0, "nb_path, ttm must be positive");
-  cudaStream_t st = current_stream();
-  ensure_pool_threshold();
-  double *d = nullptr, *d_mom = nullptr;
-  const size_t nb = sizeof(double) * (size_t)nb_path;
-  B200SV_CUDA(cudaMallocAsync(&d, 3 * nb, st));
-  B200SV_CUDA(cudaMallocAsync(&d_mom, sizeof(double) * 2, st));
-  if (use_initial_arrays) {
-    B200SV_CUDA(cudaMemcpyAsync(d, x_inout, nb, cudaMemcpyHostToDevice, st));
-    B200SV_CUDA(cudaMemcpyAsync(d + nb_path, lambda_p_inout, nb, cudaMemcpyHostToDevice, st));
-    B200SV_CUDA(cudaMemcpyAsync(d + 2 * nb_path, lambda_m_inout, nb, cudaMemcpyHostToDevice, st));
-  }
+  if (int rc = check_hawkes_flags(flags)) return rc;
   int S;
   double dt;
   time_grid(ttm, kHawkesStepsPerYear, &S, &dt);
-  int rc = launch_hawkes_slice(d, d + nb_path, d + 2 * nb_path, nb_path, 0, use_initial_arrays ? 0 : 1, *params, S, dt, slice_index, 1.0, seed, flags,
-                               d_mom, st);
-  if (rc == 0) {
-    cudaError_t e = cudaMemcpyAsync(x_inout, d, nb, cudaMemcpyDeviceToHost, st);
-    if (e == cudaSuccess) e = cudaMemcpyAsync(lambda_p_inout, d + nb_path, nb, cudaMemcpyDeviceToHost, st);
-    if (e == cudaSuccess) e = cudaMemcpyAsync(lambda_m_inout, d + 2 * nb_path, nb, cudaMemcpyDeviceToHost, st);
-    if (e != cudaSuccess) rc = fail(-2, std::string("D2H: ") + cudaGetErrorString(e));
-  }
-  cudaFreeAsync(d, st);
-  cudaFreeAsync(d_mom, st);
-  cudaError_t e = cudaStreamSynchronize(st);
-  if (rc == 0 && e != cudaSuccess) rc = fail(-2, std::string("sync: ") + cudaGetErrorString(e));
-  return rc;
+  return host_call([&](cudaStream_t st) {
+    DevBuf<double> d(st), d_mom(st);
+    B200SV_CUDA(d.alloc(3 * (size_t)nb_path));
+    B200SV_CUDA(d_mom.alloc(2));
+    if (use_initial_arrays)
+      if (int rc = state_to_device(d.p, nb_path, x_inout, lambda_p_inout, lambda_m_inout, st)) return rc;
+    if (int rc = launch_hawkes_slice(d.p, d.p + nb_path, d.p + 2 * nb_path, nb_path, 0, use_initial_arrays ? 0 : 1, *params, S, dt, slice_index, 1.0,
+                                     seed, flags, d_mom.p, st))
+      return rc;
+    return state_to_host(d.p, nb_path, x_inout, lambda_p_inout, lambda_m_inout, st);
+  });
 }
 
 int b200sv_hawkesjd_step_fixed(double* x, double* lambda_p, double* lambda_m, const double* W0, const double* U_P, const double* U_M,
                                const double* J_P, const double* J_M, int S, long long N, double dt, const b200sv_hawkes_params* params) {
   B200SV_REQUIRE(x && lambda_p && lambda_m && params && (S == 0 || (W0 && U_P && U_M && J_P && J_M)), "null pointer");
   B200SV_REQUIRE(S >= 0 && N >= 1 && dt > 0.0, "S, N, dt");
-  cudaStream_t st = current_stream();
-  ensure_pool_threshold();
-  double *d = nullptr, *w = nullptr;
-  const size_t nb = sizeof(double) * (size_t)N, wb = sizeof(double) * (size_t)N * (size_t)std::max(S, 1), wn = (size_t)N * (size_t)std::max(S, 1);
-  B200SV_CUDA(cudaMallocAsync(&d, 3 * nb, st));
-  B200SV_CUDA(cudaMallocAsync(&w, 5 * wb, st));
-  B200SV_CUDA(cudaMemcpyAsync(d, x, nb, cudaMemcpyHostToDevice, st));
-  B200SV_CUDA(cudaMemcpyAsync(d + N, lambda_p, nb, cudaMemcpyHostToDevice, st));
-  B200SV_CUDA(cudaMemcpyAsync(d + 2 * N, lambda_m, nb, cudaMemcpyHostToDevice, st));
-  const double* src[5] = {W0, U_P, U_M, J_P, J_M};
-  if (S > 0)
-    for (int k = 0; k < 5; ++k) B200SV_CUDA(cudaMemcpyAsync(w + k * wn, src[k], wb, cudaMemcpyHostToDevice, st));
-  Grid g = persistent_grid(hawkes_step_fixed_kernel, kThreads, N);
-  hawkes_step_fixed_kernel<<<g.blocks, g.threads, 0, st>>>(d, d + N, d + 2 * N, w, w + wn, w + 2 * wn, w + 3 * wn, w + 4 * wn, S, N,
-                                                            make_hawkes_consts(*params, dt));
-  int rc = check_launch("hawkes_step_fixed_kernel");
-  if (rc == 0) {
-    cudaError_t e = cudaMemcpyAsync(x, d, nb, cudaMemcpyDeviceToHost, st);
-    if (e == cudaSuccess) e = cudaMemcpyAsync(lambda_p, d + N, nb, cudaMemcpyDeviceToHost, st);
-    if (e == cudaSuccess) e = cudaMemcpyAsync(lambda_m, d + 2 * N, nb, cudaMemcpyDeviceToHost, st);
-    if (e != cudaSuccess) rc = fail(-2, std::string("D2H: ") + cudaGetErrorString(e));
-  }
-  cudaFreeAsync(d, st);
-  cudaFreeAsync(w, st);
-  cudaError_t e = cudaStreamSynchronize(st);
-  if (rc == 0 && e != cudaSuccess) rc = fail(-2, std::string("sync: ") + cudaGetErrorString(e));
-  return rc;
+  const size_t wn = (size_t)N * (size_t)std::max(S, 1);
+  return host_call([&](cudaStream_t st) {
+    DevBuf<double> d(st), w(st);
+    B200SV_CUDA(d.alloc(3 * (size_t)N));
+    B200SV_CUDA(w.alloc(5 * wn));
+    if (int rc = state_to_device(d.p, N, x, lambda_p, lambda_m, st)) return rc;
+    const double* src[5] = {W0, U_P, U_M, J_P, J_M};
+    if (S > 0)
+      for (int k = 0; k < 5; ++k) B200SV_CUDA(cudaMemcpyAsync(w.p + k * wn, src[k], sizeof(double) * wn, cudaMemcpyHostToDevice, st));
+    Grid g = persistent_grid(hawkes_step_fixed_kernel, kThreads, N);
+    hawkes_step_fixed_kernel<<<g.blocks, g.threads, 0, st>>>(d.p, d.p + N, d.p + 2 * N, w.p, w.p + wn, w.p + 2 * wn, w.p + 3 * wn, w.p + 4 * wn, S, N,
+                                                              make_hawkes_consts(*params, dt));
+    if (int rc = launched("hawkes_step_fixed_kernel")) return rc;
+    return state_to_host(d.p, N, x, lambda_p, lambda_m, st);
+  });
 }
 
 int b200sv_hawkesjd_device_draws(uint64_t seed, long long path0, long long n, int slice, int S, double dt, const b200sv_hawkes_params* params,
@@ -1913,27 +1812,23 @@ int b200sv_hawkesjd_device_draws(uint64_t seed, long long path0, long long n, in
   B200SV_REQUIRE(params && W0 && U_P && U_M && J_P && J_M && n >= 1 && S >= 1 && dt > 0.0, "null pointer / sizes");
   const int g = gauss_mode(flags);
   B200SV_REQUIRE(g == kGaussF32 || g == kGaussF64, "gauss flags");
-  cudaStream_t st = current_stream();
-  ensure_pool_threshold();
-  double* d = nullptr;
   const size_t wn = (size_t)n * S;
-  B200SV_CUDA(cudaMallocAsync(&d, sizeof(double) * 5 * wn, st));
   const HawkesConsts c = make_hawkes_consts(*params, dt);
-  const int blocks = (int)((n + 127) / 128);
-  if (g == kGaussF64)
-    hawkes_device_draws_kernel<kGaussF64><<<blocks, 128, 0, st>>>(seed, (unsigned long long)path0, n, (unsigned)slice, S, c, d, d + wn, d + 2 * wn, d + 3 * wn, d + 4 * wn);
-  else
-    hawkes_device_draws_kernel<kGaussF32><<<blocks, 128, 0, st>>>(seed, (unsigned long long)path0, n, (unsigned)slice, S, c, d, d + wn, d + 2 * wn, d + 3 * wn, d + 4 * wn);
-  int rc = check_launch("hawkes_device_draws_kernel");
-  double* dst[5] = {W0, U_P, U_M, J_P, J_M};
-  for (int k = 0; k < 5 && rc == 0; ++k) {
-    cudaError_t e = cudaMemcpyAsync(dst[k], d + k * wn, sizeof(double) * wn, cudaMemcpyDeviceToHost, st);
-    if (e != cudaSuccess) rc = fail(-2, std::string("D2H: ") + cudaGetErrorString(e));
-  }
-  cudaFreeAsync(d, st);
-  cudaError_t e = cudaStreamSynchronize(st);
-  if (rc == 0 && e != cudaSuccess) rc = fail(-2, std::string("sync: ") + cudaGetErrorString(e));
-  return rc;
+  return host_call([&](cudaStream_t st) {
+    DevBuf<double> d(st);
+    B200SV_CUDA(d.alloc(5 * wn));
+    const int blocks = (int)((n + 127) / 128);
+    if (g == kGaussF64)
+      hawkes_device_draws_kernel<kGaussF64><<<blocks, 128, 0, st>>>(seed, (unsigned long long)path0, n, (unsigned)slice, S, c, d.p, d.p + wn, d.p + 2 * wn,
+                                                                    d.p + 3 * wn, d.p + 4 * wn);
+    else
+      hawkes_device_draws_kernel<kGaussF32><<<blocks, 128, 0, st>>>(seed, (unsigned long long)path0, n, (unsigned)slice, S, c, d.p, d.p + wn, d.p + 2 * wn,
+                                                                    d.p + 3 * wn, d.p + 4 * wn);
+    if (int rc = launched("hawkes_device_draws_kernel")) return rc;
+    double* dst[5] = {W0, U_P, U_M, J_P, J_M};
+    for (int k = 0; k < 5; ++k) B200SV_CUDA(cudaMemcpyAsync(dst[k], d.p + k * wn, sizeof(double) * wn, cudaMemcpyDeviceToHost, st));
+    return 0;
+  });
 }
 
 // ---- P2P mailbox (p2p.cuh) -----------------------------------------------------------------------------------------------
@@ -2022,7 +1917,7 @@ int b200sv_dev_p2p_publish(void* ctx, const double* vals, int K, void* stream) {
   P2pCtx* c = (P2pCtx*)ctx;
   B200SV_REQUIRE(K <= c->kmax, "K exceeds the mailbox size");
   p2p_publish_kernel<<<1, 128, 0, (cudaStream_t)stream>>>(vals, K, make_publish(c, (cudaStream_t)stream));
-  return check_launch("p2p_publish_kernel");
+  return launched("p2p_publish_kernel");
 }
 
 int b200sv_dev_p2p_gather(void* ctx, int K, double* out, void* stream) {
@@ -2030,7 +1925,7 @@ int b200sv_dev_p2p_gather(void* ctx, int K, double* out, void* stream) {
   P2pCtx* c = (P2pCtx*)ctx;
   B200SV_REQUIRE(K <= c->kmax, "K exceeds the mailbox size");
   p2p_gather_kernel<<<1, 128, 0, (cudaStream_t)stream>>>(make_gather(c), K, out);
-  return check_launch("p2p_gather_kernel");
+  return launched("p2p_gather_kernel");
 }
 
 }  // extern "C"

@@ -25,8 +25,6 @@
 #include "black.cuh"
 #include "fastmath64.cuh"
 
-extern "C" void b200sv_internal_count_launch(void);
-
 namespace b200sv {
 
 struct cd {
@@ -718,6 +716,7 @@ struct SumSpec {
   double a, b;        // QVAR: a = discfactor, b = ttm ; DIGITAL: a = discfactor
   int type, slice;
 };
+static_assert(sizeof(SumSpec) <= sizeof(StrikeSpec), "the chain pricers stage either kind of spec in one StrikeSpec buffer");
 
 __global__ void __launch_bounds__(kFourierThreads) fourier_sum_kernel(const cd* __restrict__ log_mgf, const cd* __restrict__ grid, int P,
                                                                      const SumSpec* __restrict__ specs, int mode, int all_calls,
@@ -870,13 +869,6 @@ __global__ void __launch_bounds__(kFourierThreads) fourier_gamma_kernel(const cd
 // --------------------------------------------------------------------------------------------------------------------
 // host side
 // --------------------------------------------------------------------------------------------------------------------
-static int launched(const char* what) {
-  cudaError_t e = cudaGetLastError();
-  if (e != cudaSuccess) return fail(-2, std::string(what) + ": " + cudaGetErrorString(e));
-  b200sv_internal_count_launch();
-  return 0;
-}
-
 // Latency regime (few grid points in total): lane-parallel kernel; throughput regime (batches, the 40000-point psi grid): one thread per
 // point.  B200SV_MGF_LANES=0/1 overrides the choice (A/B timing in tools/bench_mgf.py).
 static bool use_lane_kernel(long long points) {
@@ -1480,20 +1472,6 @@ static bool all_half_re(const double* phi, int P) {
   return true;
 }
 
-struct DevBuf {   // RAII for stream-ordered temporaries
-  void* p = nullptr;
-  cudaStream_t st;
-  explicit DevBuf(cudaStream_t s) : st(s) {}
-  cudaError_t alloc(size_t n) { return cudaMallocAsync(&p, n ? n : 1, st); }
-  ~DevBuf() {
-    if (p) cudaFreeAsync(p, st);
-  }
-  template <typename T>
-  T* as() {
-    return (T*)p;
-  }
-};
-
 }  // namespace b200sv
 
 using namespace b200sv;
@@ -1546,44 +1524,42 @@ int b200sv_logsv_price_chain(const b200sv_logsv_params* params, int M, const dou
       ss[j - offsets[0]] = StrikeSpec{strikes[j], forwards[m], discfactors[m], (int)types[j], m, ttms[m], 0};
       qs[j - offsets[0]] = SumSpec{strikes[j] * ttms[m], discfactors[m], ttms[m], (int)types[j], m};
     }
-  cudaStream_t st = current_stream();
-  ensure_pool_threshold();
-  DevBuf d_phi(st), d_psi(st), d_spec(st), d_a(st), d_lm(st), d_ss(st), d_pr(st), d_stat(st);
-  B200SV_CUDA(d_phi.alloc(sizeof(cd) * P));
-  B200SV_CUDA(d_psi.alloc(sizeof(cd) * P));
-  if (qvar) B200SV_CUDA(cudaMemcpyAsync(d_psi.p, psi.data(), sizeof(cd) * P, cudaMemcpyHostToDevice, st));
-  B200SV_CUDA(d_spec.alloc(sizeof(ChainSpec) * M));
-  B200SV_CUDA(d_a.alloc(sizeof(cd) * (size_t)M * P * N));
-  B200SV_CUDA(d_lm.alloc(sizeof(cd) * (size_t)M * P));
-  B200SV_CUDA(d_ss.alloc(std::max(sizeof(StrikeSpec), sizeof(SumSpec)) * ss.size()));
-  B200SV_CUDA(d_pr.alloc(sizeof(double) * ss.size()));
-  B200SV_CUDA(d_stat.alloc(sizeof(int) * P));
-  B200SV_CUDA(cudaMemcpyAsync(d_phi.p, phi.data(), sizeof(cd) * P, cudaMemcpyHostToDevice, st));
-  B200SV_CUDA(cudaMemcpyAsync(d_spec.p, spec.data(), sizeof(ChainSpec) * M, cudaMemcpyHostToDevice, st));
-  if (qvar)
-    B200SV_CUDA(cudaMemcpyAsync(d_ss.p, qs.data(), sizeof(SumSpec) * qs.size(), cudaMemcpyHostToDevice, st));
-  else
-    B200SV_CUDA(cudaMemcpyAsync(d_ss.p, ss.data(), sizeof(StrikeSpec) * ss.size(), cudaMemcpyHostToDevice, st));
-  const int tpb = mgf_block_threads(P), nb = (P + tpb - 1) / tpb;
-  const double y = params->sigma0 - params->theta;
-  const cd* dpsi = qvar ? d_psi.as<cd>() : nullptr;
-  if (N == 5)
-    launch_logsv_mgf<5>(tpb, nb, st, d_phi.as<cd>(), dpsi, P, M, d_spec.as<ChainSpec>(), nullptr, d_a.as<cd>(), d_lm.as<cd>(), y, d_stat.as<int>());
-  else
-    launch_logsv_mgf<3>(tpb, nb, st, d_phi.as<cd>(), dpsi, P, M, d_spec.as<ChainSpec>(), nullptr, d_a.as<cd>(), d_lm.as<cd>(), y, d_stat.as<int>());
-  if (int rc = launched("logsv_mgf_kernel")) return rc;
-  if (Jtot > 0) {
-    if (qvar)
-      fourier_sum_kernel<<<Jtot, kFourierThreads, 0, st>>>(d_lm.as<cd>(), d_psi.as<cd>(), P, d_ss.as<SumSpec>(), kModeQvar, 0, d_pr.as<double>());
+  return host_call([&](cudaStream_t st) {
+    DevBuf<cd> d_phi(st), d_psi(st), d_a(st), d_lm(st);
+    DevBuf<ChainSpec> d_spec(st);
+    DevBuf<StrikeSpec> d_ss(st);      // the StrikeSpecs, or the (smaller) SumSpecs for Q_VAR
+    DevBuf<double> d_pr(st);
+    DevBuf<int> d_stat(st);
+    B200SV_CUDA(d_phi.upload(phi.data(), P));
+    B200SV_CUDA(qvar ? d_psi.upload(psi.data(), P) : d_psi.alloc(P));
+    B200SV_CUDA(d_spec.upload(spec.data(), M));
+    B200SV_CUDA(d_a.alloc((size_t)M * P * N));
+    B200SV_CUDA(d_lm.alloc((size_t)M * P));
+    B200SV_CUDA(d_ss.alloc(ss.size()));
+    B200SV_CUDA(d_pr.alloc(ss.size()));
+    B200SV_CUDA(d_stat.alloc(P));
+    B200SV_CUDA(qvar ? cudaMemcpyAsync(d_ss.p, qs.data(), sizeof(SumSpec) * qs.size(), cudaMemcpyHostToDevice, st)
+                     : cudaMemcpyAsync(d_ss.p, ss.data(), sizeof(StrikeSpec) * ss.size(), cudaMemcpyHostToDevice, st));
+    const int tpb = mgf_block_threads(P), nb = (P + tpb - 1) / tpb;
+    const double y = params->sigma0 - params->theta;
+    const cd* dpsi = qvar ? d_psi.p : nullptr;
+    if (N == 5)
+      launch_logsv_mgf<5>(tpb, nb, st, d_phi.p, dpsi, P, M, d_spec.p, nullptr, d_a.p, d_lm.p, y, d_stat.p);
     else
-      fourier_vanilla_kernel<<<Jtot, kFourierThreads, 0, st>>>(d_lm.as<cd>(), d_phi.as<cd>(), P, d_ss.as<StrikeSpec>(), spot ? 1 : 0, 1, d_pr.as<double>());
-    if (int rc = launched("fourier_vanilla_kernel")) return rc;
-    B200SV_CUDA(cudaMemcpyAsync(prices_out, d_pr.p, sizeof(double) * Jtot, cudaMemcpyDeviceToHost, st));
-  }
-  if (a_out) B200SV_CUDA(cudaMemcpyAsync(a_out, d_a.p, sizeof(cd) * (size_t)M * P * N, cudaMemcpyDeviceToHost, st));
-  if (log_mgf_out) B200SV_CUDA(cudaMemcpyAsync(log_mgf_out, d_lm.p, sizeof(cd) * (size_t)M * P, cudaMemcpyDeviceToHost, st));
-  B200SV_CUDA(cudaStreamSynchronize(st));
-  return 0;
+      launch_logsv_mgf<3>(tpb, nb, st, d_phi.p, dpsi, P, M, d_spec.p, nullptr, d_a.p, d_lm.p, y, d_stat.p);
+    if (int rc = launched("logsv_mgf_kernel")) return rc;
+    if (Jtot > 0) {
+      if (qvar)
+        fourier_sum_kernel<<<Jtot, kFourierThreads, 0, st>>>(d_lm.p, d_psi.p, P, (const SumSpec*)d_ss.p, kModeQvar, 0, d_pr.p);
+      else
+        fourier_vanilla_kernel<<<Jtot, kFourierThreads, 0, st>>>(d_lm.p, d_phi.p, P, d_ss.p, spot ? 1 : 0, 1, d_pr.p);
+      if (int rc = launched("fourier_vanilla_kernel")) return rc;
+      B200SV_CUDA(cudaMemcpyAsync(prices_out, d_pr.p, sizeof(double) * Jtot, cudaMemcpyDeviceToHost, st));
+    }
+    if (a_out) B200SV_CUDA(cudaMemcpyAsync(a_out, d_a.p, sizeof(cd) * (size_t)M * P * N, cudaMemcpyDeviceToHost, st));
+    if (log_mgf_out) B200SV_CUDA(cudaMemcpyAsync(log_mgf_out, d_lm.p, sizeof(cd) * (size_t)M * P, cudaMemcpyDeviceToHost, st));
+    return 0;
+  });
 }
 
 int b200sv_heston_price_chain(const b200sv_heston_params* params, int M, const double* ttms, const double* forwards,
@@ -1619,37 +1595,32 @@ int b200sv_heston_price_chain(const b200sv_heston_params* params, int M, const d
       ss[j - offsets[0]] = StrikeSpec{strikes[j], forwards[m], discfactors[m], (int)types[j], m, ttms[m], 0};
       qs[j - offsets[0]] = SumSpec{strikes[j] * ttms[m], discfactors[m], ttms[m], (int)types[j], m};
     }
-  cudaStream_t st = current_stream();
-  ensure_pool_threshold();
-  DevBuf d_phi(st), d_psi(st), d_dt(st), d_lm(st), d_ss(st), d_pr(st);
-  B200SV_CUDA(d_phi.alloc(sizeof(cd) * P));
-  B200SV_CUDA(d_psi.alloc(sizeof(cd) * P));
-  B200SV_CUDA(d_dt.alloc(sizeof(double) * M));
-  B200SV_CUDA(d_lm.alloc(sizeof(cd) * (size_t)M * P));
-  B200SV_CUDA(d_ss.alloc(std::max(sizeof(StrikeSpec), sizeof(SumSpec)) * ss.size()));
-  B200SV_CUDA(d_pr.alloc(sizeof(double) * ss.size()));
-  B200SV_CUDA(cudaMemcpyAsync(d_phi.p, phi.data(), sizeof(cd) * P, cudaMemcpyHostToDevice, st));
-  if (qvar) B200SV_CUDA(cudaMemcpyAsync(d_psi.p, psi.data(), sizeof(cd) * P, cudaMemcpyHostToDevice, st));
-  B200SV_CUDA(cudaMemcpyAsync(d_dt.p, dtaus.data(), sizeof(double) * M, cudaMemcpyHostToDevice, st));
-  if (qvar)
-    B200SV_CUDA(cudaMemcpyAsync(d_ss.p, qs.data(), sizeof(SumSpec) * qs.size(), cudaMemcpyHostToDevice, st));
-  else
-    B200SV_CUDA(cudaMemcpyAsync(d_ss.p, ss.data(), sizeof(StrikeSpec) * ss.size(), cudaMemcpyHostToDevice, st));
-  const int tpb = mgf_block_threads(P), nb = (P + tpb - 1) / tpb;
-  heston_mgf_kernel<<<nb, tpb, 0, st>>>(d_phi.as<cd>(), qvar ? d_psi.as<cd>() : nullptr, P, M, d_dt.as<double>(), *params, nullptr, nullptr,
-                                        nullptr, nullptr, d_lm.as<cd>());
-  if (int rc = launched("heston_mgf_kernel")) return rc;
-  if (Jtot > 0) {
-    if (qvar)
-      fourier_sum_kernel<<<Jtot, kFourierThreads, 0, st>>>(d_lm.as<cd>(), d_psi.as<cd>(), P, d_ss.as<SumSpec>(), kModeQvar, 0, d_pr.as<double>());
-    else
-      fourier_vanilla_kernel<<<Jtot, kFourierThreads, 0, st>>>(d_lm.as<cd>(), d_phi.as<cd>(), P, d_ss.as<StrikeSpec>(), 1, 1, d_pr.as<double>());
-    if (int rc = launched("fourier_vanilla_kernel")) return rc;
-    B200SV_CUDA(cudaMemcpyAsync(prices_out, d_pr.p, sizeof(double) * Jtot, cudaMemcpyDeviceToHost, st));
-  }
-  if (log_mgf_out) B200SV_CUDA(cudaMemcpyAsync(log_mgf_out, d_lm.p, sizeof(cd) * (size_t)M * P, cudaMemcpyDeviceToHost, st));
-  B200SV_CUDA(cudaStreamSynchronize(st));
-  return 0;
+  return host_call([&](cudaStream_t st) {
+    DevBuf<cd> d_phi(st), d_psi(st), d_lm(st);
+    DevBuf<double> d_dt(st), d_pr(st);
+    DevBuf<StrikeSpec> d_ss(st);      // the StrikeSpecs, or the (smaller) SumSpecs for Q_VAR
+    B200SV_CUDA(d_phi.upload(phi.data(), P));
+    B200SV_CUDA(qvar ? d_psi.upload(psi.data(), P) : d_psi.alloc(P));
+    B200SV_CUDA(d_dt.upload(dtaus.data(), M));
+    B200SV_CUDA(d_lm.alloc((size_t)M * P));
+    B200SV_CUDA(d_ss.alloc(ss.size()));
+    B200SV_CUDA(d_pr.alloc(ss.size()));
+    B200SV_CUDA(qvar ? cudaMemcpyAsync(d_ss.p, qs.data(), sizeof(SumSpec) * qs.size(), cudaMemcpyHostToDevice, st)
+                     : cudaMemcpyAsync(d_ss.p, ss.data(), sizeof(StrikeSpec) * ss.size(), cudaMemcpyHostToDevice, st));
+    const int tpb = mgf_block_threads(P), nb = (P + tpb - 1) / tpb;
+    heston_mgf_kernel<<<nb, tpb, 0, st>>>(d_phi.p, qvar ? d_psi.p : nullptr, P, M, d_dt.p, *params, nullptr, nullptr, nullptr, nullptr, d_lm.p);
+    if (int rc = launched("heston_mgf_kernel")) return rc;
+    if (Jtot > 0) {
+      if (qvar)
+        fourier_sum_kernel<<<Jtot, kFourierThreads, 0, st>>>(d_lm.p, d_psi.p, P, (const SumSpec*)d_ss.p, kModeQvar, 0, d_pr.p);
+      else
+        fourier_vanilla_kernel<<<Jtot, kFourierThreads, 0, st>>>(d_lm.p, d_phi.p, P, d_ss.p, 1, 1, d_pr.p);
+      if (int rc = launched("fourier_vanilla_kernel")) return rc;
+      B200SV_CUDA(cudaMemcpyAsync(prices_out, d_pr.p, sizeof(double) * Jtot, cudaMemcpyDeviceToHost, st));
+    }
+    if (log_mgf_out) B200SV_CUDA(cudaMemcpyAsync(log_mgf_out, d_lm.p, sizeof(cd) * (size_t)M * P, cudaMemcpyDeviceToHost, st));
+    return 0;
+  });
 }
 
 /* ---- batched chain pricers: B parameter sets on one chain in one pass (calibration objective + its finite-difference gradient) ---- */
@@ -1703,38 +1674,33 @@ int b200sv_logsv_price_chain_batch(const b200sv_logsv_params* params, int B, int
     yb[b] = params[b].sigma0 - params[b].theta;
     for (int m = 0; m < M; ++m) spec[(size_t)b * M + m] = ChainSpec{dtaus[m], make_model(params[b], etas ? etas[(size_t)b * M + m] : 1.0, spot)};
   }
-  cudaStream_t st = current_stream();
-  ensure_pool_threshold();
-  DevBuf d_phi(st), d_spec(st), d_y(st), d_a(st), d_lm(st), d_ss(st), d_pr(st), d_iv(st);
   const size_t nq = (size_t)B * Jtot;
-  B200SV_CUDA(d_phi.alloc(sizeof(cd) * (size_t)G * P));
-  B200SV_CUDA(d_spec.alloc(sizeof(ChainSpec) * spec.size()));
-  B200SV_CUDA(d_y.alloc(sizeof(double) * B));
-  B200SV_CUDA(d_a.alloc(sizeof(cd) * (size_t)B * M * P * N));
-  B200SV_CUDA(d_lm.alloc(sizeof(cd) * (size_t)B * M * P));
-  B200SV_CUDA(d_ss.alloc(sizeof(StrikeSpec) * nq));
-  B200SV_CUDA(d_pr.alloc(sizeof(double) * nq));
-  B200SV_CUDA(d_iv.alloc(sizeof(double) * nq));
-  B200SV_CUDA(cudaMemcpyAsync(d_phi.p, phi.data(), sizeof(cd) * (size_t)G * P, cudaMemcpyHostToDevice, st));
-  B200SV_CUDA(cudaMemcpyAsync(d_spec.p, spec.data(), sizeof(ChainSpec) * spec.size(), cudaMemcpyHostToDevice, st));
-  B200SV_CUDA(cudaMemcpyAsync(d_y.p, yb.data(), sizeof(double) * B, cudaMemcpyHostToDevice, st));
-  B200SV_CUDA(cudaMemcpyAsync(d_ss.p, ss.data(), sizeof(StrikeSpec) * nq, cudaMemcpyHostToDevice, st));
-  const long long threads = (long long)B * P;
-  const int tpb = mgf_block_threads((int)std::min<long long>(threads, 1 << 30)), nb = (P + tpb - 1) / tpb;
-  if (N == 5)
-    launch_logsv_mgf<5>(tpb, nb, st, d_phi.as<cd>(), nullptr, P, M, d_spec.as<ChainSpec>(), nullptr, d_a.as<cd>(), d_lm.as<cd>(), 0.0, nullptr, B,
-                        d_y.as<double>(), per_set_grid ? P : 0);
-  else
-    launch_logsv_mgf<3>(tpb, nb, st, d_phi.as<cd>(), nullptr, P, M, d_spec.as<ChainSpec>(), nullptr, d_a.as<cd>(), d_lm.as<cd>(), 0.0, nullptr, B,
-                        d_y.as<double>(), per_set_grid ? P : 0);
-  if (int rc = launched("logsv_mgf_kernel")) return rc;
-  fourier_vanilla_kernel<<<(unsigned)nq, kFourierThreads, 0, st>>>(d_lm.as<cd>(), d_phi.as<cd>(), P, d_ss.as<StrikeSpec>(), spot ? 1 : 0, 1,
-                                                                    d_pr.as<double>(), ivols_out ? d_iv.as<double>() : nullptr);
-  if (int rc = launched("fourier_vanilla_kernel")) return rc;
-  B200SV_CUDA(cudaMemcpyAsync(prices_out, d_pr.p, sizeof(double) * nq, cudaMemcpyDeviceToHost, st));
-  if (ivols_out) B200SV_CUDA(cudaMemcpyAsync(ivols_out, d_iv.p, sizeof(double) * nq, cudaMemcpyDeviceToHost, st));
-  B200SV_CUDA(cudaStreamSynchronize(st));
-  return 0;
+  return host_call([&](cudaStream_t st) {
+    DevBuf<cd> d_phi(st), d_a(st), d_lm(st);
+    DevBuf<ChainSpec> d_spec(st);
+    DevBuf<double> d_y(st), d_pr(st), d_iv(st);
+    DevBuf<StrikeSpec> d_ss(st);
+    B200SV_CUDA(d_phi.upload(phi.data(), (size_t)G * P));
+    B200SV_CUDA(d_spec.upload(spec.data(), spec.size()));
+    B200SV_CUDA(d_y.upload(yb.data(), B));
+    B200SV_CUDA(d_a.alloc((size_t)B * M * P * N));
+    B200SV_CUDA(d_lm.alloc((size_t)B * M * P));
+    B200SV_CUDA(d_ss.upload(ss.data(), nq));
+    B200SV_CUDA(d_pr.alloc(nq));
+    B200SV_CUDA(d_iv.alloc(nq));
+    const long long threads = (long long)B * P;
+    const int tpb = mgf_block_threads((int)std::min<long long>(threads, 1 << 30)), nb = (P + tpb - 1) / tpb;
+    if (N == 5)
+      launch_logsv_mgf<5>(tpb, nb, st, d_phi.p, nullptr, P, M, d_spec.p, nullptr, d_a.p, d_lm.p, 0.0, nullptr, B, d_y.p, per_set_grid ? P : 0);
+    else
+      launch_logsv_mgf<3>(tpb, nb, st, d_phi.p, nullptr, P, M, d_spec.p, nullptr, d_a.p, d_lm.p, 0.0, nullptr, B, d_y.p, per_set_grid ? P : 0);
+    if (int rc = launched("logsv_mgf_kernel")) return rc;
+    fourier_vanilla_kernel<<<(unsigned)nq, kFourierThreads, 0, st>>>(d_lm.p, d_phi.p, P, d_ss.p, spot ? 1 : 0, 1, d_pr.p, ivols_out ? d_iv.p : nullptr);
+    if (int rc = launched("fourier_vanilla_kernel")) return rc;
+    B200SV_CUDA(cudaMemcpyAsync(prices_out, d_pr.p, sizeof(double) * nq, cudaMemcpyDeviceToHost, st));
+    if (ivols_out) B200SV_CUDA(cudaMemcpyAsync(ivols_out, d_iv.p, sizeof(double) * nq, cudaMemcpyDeviceToHost, st));
+    return 0;
+  });
 }
 
 int b200sv_heston_price_chain_batch(const b200sv_heston_params* params, int B, int M, const double* ttms, const double* forwards,
@@ -1753,32 +1719,29 @@ int b200sv_heston_price_chain_batch(const b200sv_heston_params* params, int B, i
     build_phi(per_set_grid ? std::min(0.3, std::sqrt(params[g].v0 * ttms[0])) : vol_scaler, true, P, one);
     phi.insert(phi.end(), one.begin(), one.end());
   }
-  cudaStream_t st = current_stream();
-  ensure_pool_threshold();
-  DevBuf d_phi(st), d_hp(st), d_dt(st), d_lm(st), d_ss(st), d_pr(st), d_iv(st);
   const size_t nq = (size_t)B * Jtot;
-  B200SV_CUDA(d_phi.alloc(sizeof(cd) * (size_t)G * P));
-  B200SV_CUDA(d_hp.alloc(sizeof(b200sv_heston_params) * B));
-  B200SV_CUDA(d_dt.alloc(sizeof(double) * M));
-  B200SV_CUDA(d_lm.alloc(sizeof(cd) * (size_t)B * M * P));
-  B200SV_CUDA(d_ss.alloc(sizeof(StrikeSpec) * nq));
-  B200SV_CUDA(d_pr.alloc(sizeof(double) * nq));
-  B200SV_CUDA(d_iv.alloc(sizeof(double) * nq));
-  B200SV_CUDA(cudaMemcpyAsync(d_phi.p, phi.data(), sizeof(cd) * (size_t)G * P, cudaMemcpyHostToDevice, st));
-  B200SV_CUDA(cudaMemcpyAsync(d_hp.p, params, sizeof(b200sv_heston_params) * B, cudaMemcpyHostToDevice, st));
-  B200SV_CUDA(cudaMemcpyAsync(d_dt.p, dtaus.data(), sizeof(double) * M, cudaMemcpyHostToDevice, st));
-  B200SV_CUDA(cudaMemcpyAsync(d_ss.p, ss.data(), sizeof(StrikeSpec) * nq, cudaMemcpyHostToDevice, st));
-  const int tpb = 64, nb = (P + tpb - 1) / tpb;
-  heston_mgf_kernel<<<dim3(nb, B), tpb, 0, st>>>(d_phi.as<cd>(), nullptr, P, M, d_dt.as<double>(), params[0], nullptr, nullptr, nullptr, nullptr,
-                                                 d_lm.as<cd>(), d_hp.as<b200sv_heston_params>(), per_set_grid ? P : 0);
-  if (int rc = launched("heston_mgf_kernel")) return rc;
-  fourier_vanilla_kernel<<<(unsigned)nq, kFourierThreads, 0, st>>>(d_lm.as<cd>(), d_phi.as<cd>(), P, d_ss.as<StrikeSpec>(), 1, 1, d_pr.as<double>(),
-                                                                    ivols_out ? d_iv.as<double>() : nullptr);
-  if (int rc = launched("fourier_vanilla_kernel")) return rc;
-  B200SV_CUDA(cudaMemcpyAsync(prices_out, d_pr.p, sizeof(double) * nq, cudaMemcpyDeviceToHost, st));
-  if (ivols_out) B200SV_CUDA(cudaMemcpyAsync(ivols_out, d_iv.p, sizeof(double) * nq, cudaMemcpyDeviceToHost, st));
-  B200SV_CUDA(cudaStreamSynchronize(st));
-  return 0;
+  return host_call([&](cudaStream_t st) {
+    DevBuf<cd> d_phi(st), d_lm(st);
+    DevBuf<b200sv_heston_params> d_hp(st);
+    DevBuf<double> d_dt(st), d_pr(st), d_iv(st);
+    DevBuf<StrikeSpec> d_ss(st);
+    B200SV_CUDA(d_phi.upload(phi.data(), (size_t)G * P));
+    B200SV_CUDA(d_hp.upload(params, B));
+    B200SV_CUDA(d_dt.upload(dtaus.data(), M));
+    B200SV_CUDA(d_lm.alloc((size_t)B * M * P));
+    B200SV_CUDA(d_ss.upload(ss.data(), nq));
+    B200SV_CUDA(d_pr.alloc(nq));
+    B200SV_CUDA(d_iv.alloc(nq));
+    const int tpb = 64, nb = (P + tpb - 1) / tpb;
+    heston_mgf_kernel<<<dim3(nb, B), tpb, 0, st>>>(d_phi.p, nullptr, P, M, d_dt.p, params[0], nullptr, nullptr, nullptr, nullptr, d_lm.p, d_hp.p,
+                                                   per_set_grid ? P : 0);
+    if (int rc = launched("heston_mgf_kernel")) return rc;
+    fourier_vanilla_kernel<<<(unsigned)nq, kFourierThreads, 0, st>>>(d_lm.p, d_phi.p, P, d_ss.p, 1, 1, d_pr.p, ivols_out ? d_iv.p : nullptr);
+    if (int rc = launched("fourier_vanilla_kernel")) return rc;
+    B200SV_CUDA(cudaMemcpyAsync(prices_out, d_pr.p, sizeof(double) * nq, cudaMemcpyDeviceToHost, st));
+    if (ivols_out) B200SV_CUDA(cudaMemcpyAsync(ivols_out, d_iv.p, sizeof(double) * nq, cudaMemcpyDeviceToHost, st));
+    return 0;
+  });
 }
 
 /* Hawkes jump-diffusion Fourier chain (hawkesjd_chain_pricer / hawkesjd_chain_pricer_with_risk_premia, hawkes_jd_pricer.py:365-515).
@@ -1802,76 +1765,75 @@ int b200sv_hawkesjd_price_chain(const b200sv_hawkes_params* params, int M, const
   } else if (int rc = check_fourier_types(types + offsets[0], Jtot, spot)) {
     return rc;
   }
-  std::vector<double> dtaus(M);
+  std::vector<double> dts(2 * (size_t)M);                                      // [increments | full maturities]
   double t0 = 0.0, tmin = ttms[0];
   for (int m = 0; m < M; ++m) {
     B200SV_REQUIRE(ttms[m] > t0, "ttms must be positive and strictly increasing");
-    dtaus[m] = ttms[m] - t0;
+    dts[m] = ttms[m] - t0;
+    dts[M + m] = ttms[m];
     t0 = ttms[m];
     tmin = std::min(tmin, ttms[m]);
   }
+  for (int m = 0; m < M; ++m)
+    for (int j = offsets[m]; j < offsets[m + 1]; ++j) B200SV_REQUIRE(strikes[j] > 0.0, "strikes must be positive");
   if (!(vol_scaler > 0.0)) vol_scaler = std::min(std::max(params->sigma, 0.2), 0.5) * std::sqrt(std::min(tmin, 1.0 / 12.0));   // :360-362
   std::vector<double> phi;
   build_phi(vol_scaler, true, P, phi);                                         // get_transform_var_grid default is_spot_measure=True (:385)
   if (with_gamma)
     for (int i = 0; i < P; ++i) phi[2 * i] = -0.5 - risk_premia_gamma;           // real_phi (:451)
   const HawkesMgfConsts c = make_hawkes_mgf_consts(*params);
-  cudaStream_t st = current_stream();
-  ensure_pool_threshold();
-  DevBuf d_phi(st), d_dt(st), d_a(st), d_lm(st), d_ss(st), d_pr(st), d_g(st);
-  B200SV_CUDA(d_phi.alloc(sizeof(cd) * P));
-  B200SV_CUDA(d_dt.alloc(sizeof(double) * 2 * M));
-  B200SV_CUDA(d_a.alloc(sizeof(cd) * (size_t)M * P * 3));
-  B200SV_CUDA(d_lm.alloc(sizeof(cd) * (size_t)M * P));
-  B200SV_CUDA(cudaMemcpyAsync(d_phi.p, phi.data(), sizeof(cd) * P, cudaMemcpyHostToDevice, st));
-  std::vector<double> dts(dtaus);
-  dts.insert(dts.end(), ttms, ttms + M);                                        // [increments | full maturities]
-  B200SV_CUDA(cudaMemcpyAsync(d_dt.p, dts.data(), sizeof(double) * 2 * M, cudaMemcpyHostToDevice, st));
   std::vector<double> normalizers(M, 1.0), gamma_forwards(M, 1.0);
-  if (with_gamma) {                                                            // hawkesjd_forwards_under_risk_kernel (:487-515)
-    const double two[4] = {-risk_premia_gamma, 0.0, -risk_premia_gamma - 1.0, 0.0};
-    B200SV_CUDA(d_g.alloc(sizeof(cd) * (2 + 2 * (size_t)M)));
-    B200SV_CUDA(cudaMemcpyAsync(d_g.p, two, sizeof(two), cudaMemcpyHostToDevice, st));
-    hawkes_mgf_kernel<4><<<1, 4, 0, st>>>(d_g.as<cd>(), nullptr, 2, M, d_dt.as<double>() + M, c, nullptr, nullptr, d_g.as<cd>() + 2, 1, nullptr);
+  const int rc = host_call([&](cudaStream_t st) {
+    DevBuf<cd> d_phi(st), d_a(st), d_lm(st), d_g(st);
+    DevBuf<double> d_dt(st), d_pr(st);
+    DevBuf<StrikeSpec> d_ss(st);
+    B200SV_CUDA(d_phi.upload(phi.data(), P));
+    B200SV_CUDA(d_dt.upload(dts.data(), 2 * (size_t)M));
+    B200SV_CUDA(d_a.alloc((size_t)M * P * 3));
+    B200SV_CUDA(d_lm.alloc((size_t)M * P));
+    if (with_gamma) {                                                            // hawkesjd_forwards_under_risk_kernel (:487-515)
+      const double two[4] = {-risk_premia_gamma, 0.0, -risk_premia_gamma - 1.0, 0.0};
+      B200SV_CUDA(d_g.alloc(2 + 2 * (size_t)M));
+      B200SV_CUDA(cudaMemcpyAsync(d_g.p, two, sizeof(two), cudaMemcpyHostToDevice, st));
+      hawkes_mgf_kernel<4><<<1, 4, 0, st>>>(d_g.p, nullptr, 2, M, d_dt.p + M, c, nullptr, nullptr, d_g.p + 2, 1, nullptr);
+      if (int rc = launched("hawkes_mgf_kernel")) return rc;
+      std::vector<double> lm2(4 * (size_t)M);
+      B200SV_CUDA(cudaMemcpyAsync(lm2.data(), d_g.p + 2, sizeof(cd) * 2 * M, cudaMemcpyDeviceToHost, st));
+      B200SV_CUDA(cudaStreamSynchronize(st));                                    // the strike specs below need these on the host
+      for (int m = 0; m < M; ++m) {                                              // log_mgf layout [m][point]
+        normalizers[m] = 1.0 / std::exp(lm2[2 * (2 * (size_t)m + 0)]);
+        gamma_forwards[m] = forwards[m] * std::exp(lm2[2 * (2 * (size_t)m + 1)]) * normalizers[m];
+      }
+    }
+    std::vector<StrikeSpec> ss(std::max(Jtot, 1));
+    for (int m = 0; m < M; ++m)
+      for (int j = offsets[m]; j < offsets[m + 1]; ++j)
+        ss[j - offsets[0]] = with_gamma ? StrikeSpec{strikes[j], forwards[m], normalizers[m], (int)types[j], m, gamma_forwards[m], 0}
+                                        : StrikeSpec{strikes[j], forwards[m], discfactors[m], (int)types[j], m, ttms[m], 0};
+    B200SV_CUDA(d_ss.upload(ss.data(), ss.size()));
+    B200SV_CUDA(d_pr.alloc(ss.size()));
+    const int tpb = mgf_block_threads(P), nb = (P + tpb - 1) / tpb;
+    switch (tpb) {
+      case 4: hawkes_mgf_kernel<4><<<nb, 4, 0, st>>>(d_phi.p, nullptr, P, M, d_dt.p, c, nullptr, d_a.p, d_lm.p, 0, nullptr); break;
+      case 8: hawkes_mgf_kernel<8><<<nb, 8, 0, st>>>(d_phi.p, nullptr, P, M, d_dt.p, c, nullptr, d_a.p, d_lm.p, 0, nullptr); break;
+      case 16: hawkes_mgf_kernel<16><<<nb, 16, 0, st>>>(d_phi.p, nullptr, P, M, d_dt.p, c, nullptr, d_a.p, d_lm.p, 0, nullptr); break;
+      case 32: hawkes_mgf_kernel<32><<<nb, 32, 0, st>>>(d_phi.p, nullptr, P, M, d_dt.p, c, nullptr, d_a.p, d_lm.p, 0, nullptr); break;
+      default: hawkes_mgf_kernel<64><<<nb, 64, 0, st>>>(d_phi.p, nullptr, P, M, d_dt.p, c, nullptr, d_a.p, d_lm.p, 0, nullptr); break;
+    }
     if (int rc = launched("hawkes_mgf_kernel")) return rc;
-    std::vector<double> lm2(4 * (size_t)M);
-    B200SV_CUDA(cudaMemcpyAsync(lm2.data(), d_g.as<cd>() + 2, sizeof(cd) * 2 * M, cudaMemcpyDeviceToHost, st));
-    B200SV_CUDA(cudaStreamSynchronize(st));
-    for (int m = 0; m < M; ++m) {                                              // log_mgf layout [m][point]
-      normalizers[m] = 1.0 / std::exp(lm2[2 * (2 * (size_t)m + 0)]);
-      gamma_forwards[m] = forwards[m] * std::exp(lm2[2 * (2 * (size_t)m + 1)]) * normalizers[m];
+    if (Jtot > 0) {
+      if (with_gamma)
+        fourier_gamma_kernel<<<Jtot, kFourierThreads, 0, st>>>(d_lm.p, d_phi.p, P, d_ss.p, risk_premia_gamma, d_pr.p);
+      else
+        fourier_vanilla_kernel<<<Jtot, kFourierThreads, 0, st>>>(d_lm.p, d_phi.p, P, d_ss.p, spot ? 1 : 0, 1, d_pr.p);
+      if (int rc = launched("fourier kernel")) return rc;
+      B200SV_CUDA(cudaMemcpyAsync(prices_out, d_pr.p, sizeof(double) * Jtot, cudaMemcpyDeviceToHost, st));
     }
-  }
-  std::vector<StrikeSpec> ss(std::max(Jtot, 1));
-  for (int m = 0; m < M; ++m)
-    for (int j = offsets[m]; j < offsets[m + 1]; ++j) {
-      B200SV_REQUIRE(strikes[j] > 0.0, "strikes must be positive");
-      ss[j - offsets[0]] = with_gamma ? StrikeSpec{strikes[j], forwards[m], normalizers[m], (int)types[j], m, gamma_forwards[m], 0}
-                                      : StrikeSpec{strikes[j], forwards[m], discfactors[m], (int)types[j], m, ttms[m], 0};
-    }
-  B200SV_CUDA(d_ss.alloc(sizeof(StrikeSpec) * ss.size()));
-  B200SV_CUDA(d_pr.alloc(sizeof(double) * ss.size()));
-  B200SV_CUDA(cudaMemcpyAsync(d_ss.p, ss.data(), sizeof(StrikeSpec) * ss.size(), cudaMemcpyHostToDevice, st));
-  const int tpb = mgf_block_threads(P), nb = (P + tpb - 1) / tpb;
-  switch (tpb) {
-    case 4: hawkes_mgf_kernel<4><<<nb, 4, 0, st>>>(d_phi.as<cd>(), nullptr, P, M, d_dt.as<double>(), c, nullptr, d_a.as<cd>(), d_lm.as<cd>(), 0, nullptr); break;
-    case 8: hawkes_mgf_kernel<8><<<nb, 8, 0, st>>>(d_phi.as<cd>(), nullptr, P, M, d_dt.as<double>(), c, nullptr, d_a.as<cd>(), d_lm.as<cd>(), 0, nullptr); break;
-    case 16: hawkes_mgf_kernel<16><<<nb, 16, 0, st>>>(d_phi.as<cd>(), nullptr, P, M, d_dt.as<double>(), c, nullptr, d_a.as<cd>(), d_lm.as<cd>(), 0, nullptr); break;
-    case 32: hawkes_mgf_kernel<32><<<nb, 32, 0, st>>>(d_phi.as<cd>(), nullptr, P, M, d_dt.as<double>(), c, nullptr, d_a.as<cd>(), d_lm.as<cd>(), 0, nullptr); break;
-    default: hawkes_mgf_kernel<64><<<nb, 64, 0, st>>>(d_phi.as<cd>(), nullptr, P, M, d_dt.as<double>(), c, nullptr, d_a.as<cd>(), d_lm.as<cd>(), 0, nullptr); break;
-  }
-  if (int rc = launched("hawkes_mgf_kernel")) return rc;
-  if (Jtot > 0) {
-    if (with_gamma)
-      fourier_gamma_kernel<<<Jtot, kFourierThreads, 0, st>>>(d_lm.as<cd>(), d_phi.as<cd>(), P, d_ss.as<StrikeSpec>(), risk_premia_gamma, d_pr.as<double>());
-    else
-      fourier_vanilla_kernel<<<Jtot, kFourierThreads, 0, st>>>(d_lm.as<cd>(), d_phi.as<cd>(), P, d_ss.as<StrikeSpec>(), spot ? 1 : 0, 1, d_pr.as<double>());
-    if (int rc = launched("fourier kernel")) return rc;
-    B200SV_CUDA(cudaMemcpyAsync(prices_out, d_pr.p, sizeof(double) * Jtot, cudaMemcpyDeviceToHost, st));
-  }
-  if (a_out) B200SV_CUDA(cudaMemcpyAsync(a_out, d_a.p, sizeof(cd) * (size_t)M * P * 3, cudaMemcpyDeviceToHost, st));
-  if (log_mgf_out) B200SV_CUDA(cudaMemcpyAsync(log_mgf_out, d_lm.p, sizeof(cd) * (size_t)M * P, cudaMemcpyDeviceToHost, st));
-  B200SV_CUDA(cudaStreamSynchronize(st));
+    if (a_out) B200SV_CUDA(cudaMemcpyAsync(a_out, d_a.p, sizeof(cd) * (size_t)M * P * 3, cudaMemcpyDeviceToHost, st));
+    if (log_mgf_out) B200SV_CUDA(cudaMemcpyAsync(log_mgf_out, d_lm.p, sizeof(cd) * (size_t)M * P, cudaMemcpyDeviceToHost, st));
+    return 0;
+  });
+  if (rc) return rc;
   if (normalizers_out) std::copy(normalizers.begin(), normalizers.end(), normalizers_out);
   if (gamma_forwards_out) std::copy(gamma_forwards.begin(), gamma_forwards.end(), gamma_forwards_out);
   return 0;
@@ -1883,33 +1845,29 @@ int b200sv_hawkesjd_mgf_grid(const double* phi, const double* psi, int P, double
   B200SV_REQUIRE(phi && a_inout && params && log_mgf_out, "null pointer");
   B200SV_REQUIRE(P >= 1 && dtau > 0.0, "P >= 1, dtau > 0");
   const HawkesMgfConsts c = make_hawkes_mgf_consts(*params);
-  cudaStream_t st = current_stream();
-  ensure_pool_threshold();
-  DevBuf d_phi(st), d_psi(st), d_dt(st), d_a0(st), d_a1(st), d_lm(st);
-  B200SV_CUDA(d_phi.alloc(sizeof(cd) * P));
-  B200SV_CUDA(d_psi.alloc(sizeof(cd) * P));
-  B200SV_CUDA(d_dt.alloc(sizeof(double)));
-  B200SV_CUDA(d_a0.alloc(sizeof(cd) * (size_t)P * 3));
-  B200SV_CUDA(d_a1.alloc(sizeof(cd) * (size_t)P * 3));
-  B200SV_CUDA(d_lm.alloc(sizeof(cd) * P));
-  B200SV_CUDA(cudaMemcpyAsync(d_phi.p, phi, sizeof(cd) * P, cudaMemcpyHostToDevice, st));
-  if (psi) B200SV_CUDA(cudaMemcpyAsync(d_psi.p, psi, sizeof(cd) * P, cudaMemcpyHostToDevice, st));
-  B200SV_CUDA(cudaMemcpyAsync(d_dt.p, &dtau, sizeof(double), cudaMemcpyHostToDevice, st));
-  B200SV_CUDA(cudaMemcpyAsync(d_a0.p, a_inout, sizeof(cd) * (size_t)P * 3, cudaMemcpyHostToDevice, st));
-  const cd* dpsi = psi ? d_psi.as<cd>() : nullptr;
-  const int tpb = mgf_block_threads(P), nb = (P + tpb - 1) / tpb;
-  switch (tpb) {
-    case 4: hawkes_mgf_kernel<4><<<nb, 4, 0, st>>>(d_phi.as<cd>(), dpsi, P, 1, d_dt.as<double>(), c, d_a0.as<cd>(), d_a1.as<cd>(), d_lm.as<cd>(), 0, nullptr); break;
-    case 8: hawkes_mgf_kernel<8><<<nb, 8, 0, st>>>(d_phi.as<cd>(), dpsi, P, 1, d_dt.as<double>(), c, d_a0.as<cd>(), d_a1.as<cd>(), d_lm.as<cd>(), 0, nullptr); break;
-    case 16: hawkes_mgf_kernel<16><<<nb, 16, 0, st>>>(d_phi.as<cd>(), dpsi, P, 1, d_dt.as<double>(), c, d_a0.as<cd>(), d_a1.as<cd>(), d_lm.as<cd>(), 0, nullptr); break;
-    case 32: hawkes_mgf_kernel<32><<<nb, 32, 0, st>>>(d_phi.as<cd>(), dpsi, P, 1, d_dt.as<double>(), c, d_a0.as<cd>(), d_a1.as<cd>(), d_lm.as<cd>(), 0, nullptr); break;
-    default: hawkes_mgf_kernel<64><<<nb, 64, 0, st>>>(d_phi.as<cd>(), dpsi, P, 1, d_dt.as<double>(), c, d_a0.as<cd>(), d_a1.as<cd>(), d_lm.as<cd>(), 0, nullptr); break;
-  }
-  if (int rc = launched("hawkes_mgf_kernel")) return rc;
-  B200SV_CUDA(cudaMemcpyAsync(a_inout, d_a1.p, sizeof(cd) * (size_t)P * 3, cudaMemcpyDeviceToHost, st));
-  B200SV_CUDA(cudaMemcpyAsync(log_mgf_out, d_lm.p, sizeof(cd) * P, cudaMemcpyDeviceToHost, st));
-  B200SV_CUDA(cudaStreamSynchronize(st));
-  return 0;
+  return host_call([&](cudaStream_t st) {
+    DevBuf<cd> d_phi(st), d_psi(st), d_a0(st), d_a1(st), d_lm(st);
+    DevBuf<double> d_dt(st);
+    B200SV_CUDA(d_phi.upload(phi, P));
+    B200SV_CUDA(psi ? d_psi.upload(psi, P) : d_psi.alloc(P));
+    B200SV_CUDA(d_dt.upload(&dtau, 1));
+    B200SV_CUDA(d_a0.upload(a_inout, (size_t)P * 3));
+    B200SV_CUDA(d_a1.alloc((size_t)P * 3));
+    B200SV_CUDA(d_lm.alloc(P));
+    const cd* dpsi = psi ? d_psi.p : nullptr;
+    const int tpb = mgf_block_threads(P), nb = (P + tpb - 1) / tpb;
+    switch (tpb) {
+      case 4: hawkes_mgf_kernel<4><<<nb, 4, 0, st>>>(d_phi.p, dpsi, P, 1, d_dt.p, c, d_a0.p, d_a1.p, d_lm.p, 0, nullptr); break;
+      case 8: hawkes_mgf_kernel<8><<<nb, 8, 0, st>>>(d_phi.p, dpsi, P, 1, d_dt.p, c, d_a0.p, d_a1.p, d_lm.p, 0, nullptr); break;
+      case 16: hawkes_mgf_kernel<16><<<nb, 16, 0, st>>>(d_phi.p, dpsi, P, 1, d_dt.p, c, d_a0.p, d_a1.p, d_lm.p, 0, nullptr); break;
+      case 32: hawkes_mgf_kernel<32><<<nb, 32, 0, st>>>(d_phi.p, dpsi, P, 1, d_dt.p, c, d_a0.p, d_a1.p, d_lm.p, 0, nullptr); break;
+      default: hawkes_mgf_kernel<64><<<nb, 64, 0, st>>>(d_phi.p, dpsi, P, 1, d_dt.p, c, d_a0.p, d_a1.p, d_lm.p, 0, nullptr); break;
+    }
+    if (int rc = launched("hawkes_mgf_kernel")) return rc;
+    B200SV_CUDA(cudaMemcpyAsync(a_inout, d_a1.p, sizeof(cd) * (size_t)P * 3, cudaMemcpyDeviceToHost, st));
+    B200SV_CUDA(cudaMemcpyAsync(log_mgf_out, d_lm.p, sizeof(cd) * P, cudaMemcpyDeviceToHost, st));
+    return 0;
+  });
 }
 
 int b200sv_logsv_mgf_grid(const double* phi, const double* psi, int P, double dtau, double* a_inout,
@@ -1921,31 +1879,27 @@ int b200sv_logsv_mgf_grid(const double* phi, const double* psi, int P, double dt
     return fail(-4, "expansion_order not implemented");
   const int N = expansion_order == B200SV_ORDER_FIRST ? 3 : 5;
   ChainSpec spec{dtau, make_model(*params, eta, is_spot_measure != 0)};
-  cudaStream_t st = current_stream();
-  ensure_pool_threshold();
-  DevBuf d_phi(st), d_psi(st), d_spec(st), d_a0(st), d_a1(st), d_lm(st);
-  B200SV_CUDA(d_phi.alloc(sizeof(cd) * P));
-  B200SV_CUDA(d_psi.alloc(sizeof(cd) * P));
-  B200SV_CUDA(d_spec.alloc(sizeof(ChainSpec)));
-  B200SV_CUDA(d_a0.alloc(sizeof(cd) * (size_t)P * N));
-  B200SV_CUDA(d_a1.alloc(sizeof(cd) * (size_t)P * N));
-  B200SV_CUDA(d_lm.alloc(sizeof(cd) * P));
-  B200SV_CUDA(cudaMemcpyAsync(d_phi.p, phi, sizeof(cd) * P, cudaMemcpyHostToDevice, st));
-  if (psi) B200SV_CUDA(cudaMemcpyAsync(d_psi.p, psi, sizeof(cd) * P, cudaMemcpyHostToDevice, st));
-  B200SV_CUDA(cudaMemcpyAsync(d_spec.p, &spec, sizeof(ChainSpec), cudaMemcpyHostToDevice, st));
-  B200SV_CUDA(cudaMemcpyAsync(d_a0.p, a_inout, sizeof(cd) * (size_t)P * N, cudaMemcpyHostToDevice, st));
-  const int tpb = mgf_block_threads(P), nb = (P + tpb - 1) / tpb;
-  const double y = params->sigma0 - params->theta;
-  const cd* dpsi = psi ? d_psi.as<cd>() : nullptr;
-  if (N == 5)
-    launch_logsv_mgf<5>(tpb, nb, st, d_phi.as<cd>(), dpsi, P, 1, d_spec.as<ChainSpec>(), d_a0.as<cd>(), d_a1.as<cd>(), d_lm.as<cd>(), y, nullptr);
-  else
-    launch_logsv_mgf<3>(tpb, nb, st, d_phi.as<cd>(), dpsi, P, 1, d_spec.as<ChainSpec>(), d_a0.as<cd>(), d_a1.as<cd>(), d_lm.as<cd>(), y, nullptr);
-  if (int rc = launched("logsv_mgf_kernel")) return rc;
-  B200SV_CUDA(cudaMemcpyAsync(a_inout, d_a1.p, sizeof(cd) * (size_t)P * N, cudaMemcpyDeviceToHost, st));
-  B200SV_CUDA(cudaMemcpyAsync(log_mgf_out, d_lm.p, sizeof(cd) * P, cudaMemcpyDeviceToHost, st));
-  B200SV_CUDA(cudaStreamSynchronize(st));
-  return 0;
+  return host_call([&](cudaStream_t st) {
+    DevBuf<cd> d_phi(st), d_psi(st), d_a0(st), d_a1(st), d_lm(st);
+    DevBuf<ChainSpec> d_spec(st);
+    B200SV_CUDA(d_phi.upload(phi, P));
+    B200SV_CUDA(psi ? d_psi.upload(psi, P) : d_psi.alloc(P));
+    B200SV_CUDA(d_spec.upload(&spec, 1));
+    B200SV_CUDA(d_a0.upload(a_inout, (size_t)P * N));
+    B200SV_CUDA(d_a1.alloc((size_t)P * N));
+    B200SV_CUDA(d_lm.alloc(P));
+    const int tpb = mgf_block_threads(P), nb = (P + tpb - 1) / tpb;
+    const double y = params->sigma0 - params->theta;
+    const cd* dpsi = psi ? d_psi.p : nullptr;
+    if (N == 5)
+      launch_logsv_mgf<5>(tpb, nb, st, d_phi.p, dpsi, P, 1, d_spec.p, d_a0.p, d_a1.p, d_lm.p, y, nullptr);
+    else
+      launch_logsv_mgf<3>(tpb, nb, st, d_phi.p, dpsi, P, 1, d_spec.p, d_a0.p, d_a1.p, d_lm.p, y, nullptr);
+    if (int rc = launched("logsv_mgf_kernel")) return rc;
+    B200SV_CUDA(cudaMemcpyAsync(a_inout, d_a1.p, sizeof(cd) * (size_t)P * N, cudaMemcpyDeviceToHost, st));
+    B200SV_CUDA(cudaMemcpyAsync(log_mgf_out, d_lm.p, sizeof(cd) * P, cudaMemcpyDeviceToHost, st));
+    return 0;
+  });
 }
 
 // func_a_ode_quadratic_terms (pricers/logsv/affine_expansion.py:67-184) for a grid of transform points: the dense tensors the reference
@@ -1959,28 +1913,25 @@ int b200sv_logsv_ode_terms(const double* phi, const double* psi, int P, const b2
   if (expansion_order != B200SV_ORDER_FIRST && expansion_order != B200SV_ORDER_SECOND) return fail(-4, "expansion_order not implemented");
   const int N = expansion_order == B200SV_ORDER_FIRST ? 3 : 5;
   const LogsvModel model = make_model(*params, eta, is_spot_measure != 0);
-  cudaStream_t st = current_stream();
-  ensure_pool_threshold();
-  DevBuf d_phi(st), d_psi(st), d_M(st), d_L(st), d_H(st);
-  const size_t nM = (size_t)P * N * N * N, nL = (size_t)P * N * N, nH = (size_t)P * N;
-  B200SV_CUDA(d_phi.alloc(sizeof(cd) * P));
-  B200SV_CUDA(d_psi.alloc(sizeof(cd) * P));
-  B200SV_CUDA(d_M.alloc(sizeof(cd) * nM));
-  B200SV_CUDA(d_L.alloc(sizeof(cd) * nL));
-  B200SV_CUDA(d_H.alloc(sizeof(cd) * nH));
-  B200SV_CUDA(cudaMemcpyAsync(d_phi.p, phi, sizeof(cd) * P, cudaMemcpyHostToDevice, st));
-  if (psi) B200SV_CUDA(cudaMemcpyAsync(d_psi.p, psi, sizeof(cd) * P, cudaMemcpyHostToDevice, st));
-  const cd* dpsi = psi ? d_psi.as<cd>() : nullptr;
-  if (N == 5)
-    logsv_ode_terms_kernel<5><<<(P + 63) / 64, 64, 0, st>>>(d_phi.as<cd>(), dpsi, P, model, d_M.as<cd>(), d_L.as<cd>(), d_H.as<cd>());
-  else
-    logsv_ode_terms_kernel<3><<<(P + 63) / 64, 64, 0, st>>>(d_phi.as<cd>(), dpsi, P, model, d_M.as<cd>(), d_L.as<cd>(), d_H.as<cd>());
-  if (int rc = launched("logsv_ode_terms_kernel")) return rc;
-  B200SV_CUDA(cudaMemcpyAsync(M_out, d_M.p, sizeof(cd) * nM, cudaMemcpyDeviceToHost, st));
-  B200SV_CUDA(cudaMemcpyAsync(L_out, d_L.p, sizeof(cd) * nL, cudaMemcpyDeviceToHost, st));
-  B200SV_CUDA(cudaMemcpyAsync(H_out, d_H.p, sizeof(cd) * nH, cudaMemcpyDeviceToHost, st));
-  B200SV_CUDA(cudaStreamSynchronize(st));
-  return 0;
+  return host_call([&](cudaStream_t st) {
+    DevBuf<cd> d_phi(st), d_psi(st), d_M(st), d_L(st), d_H(st);
+    const size_t nM = (size_t)P * N * N * N, nL = (size_t)P * N * N, nH = (size_t)P * N;
+    B200SV_CUDA(d_phi.upload(phi, P));
+    B200SV_CUDA(psi ? d_psi.upload(psi, P) : d_psi.alloc(P));
+    B200SV_CUDA(d_M.alloc(nM));
+    B200SV_CUDA(d_L.alloc(nL));
+    B200SV_CUDA(d_H.alloc(nH));
+    const cd* dpsi = psi ? d_psi.p : nullptr;
+    if (N == 5)
+      logsv_ode_terms_kernel<5><<<(P + 63) / 64, 64, 0, st>>>(d_phi.p, dpsi, P, model, d_M.p, d_L.p, d_H.p);
+    else
+      logsv_ode_terms_kernel<3><<<(P + 63) / 64, 64, 0, st>>>(d_phi.p, dpsi, P, model, d_M.p, d_L.p, d_H.p);
+    if (int rc = launched("logsv_ode_terms_kernel")) return rc;
+    B200SV_CUDA(cudaMemcpyAsync(M_out, d_M.p, sizeof(cd) * nM, cudaMemcpyDeviceToHost, st));
+    B200SV_CUDA(cudaMemcpyAsync(L_out, d_L.p, sizeof(cd) * nL, cudaMemcpyDeviceToHost, st));
+    B200SV_CUDA(cudaMemcpyAsync(H_out, d_H.p, sizeof(cd) * nH, cudaMemcpyDeviceToHost, st));
+    return 0;
+  });
 }
 
 int b200sv_logsv_ode_rhs(const double* phi, const double* psi, int P, const double* A, const b200sv_logsv_params* params, double eta,
@@ -1990,47 +1941,38 @@ int b200sv_logsv_ode_rhs(const double* phi, const double* psi, int P, const doub
   if (expansion_order != B200SV_ORDER_FIRST && expansion_order != B200SV_ORDER_SECOND) return fail(-4, "expansion_order not implemented");
   const int N = expansion_order == B200SV_ORDER_FIRST ? 3 : 5;
   const LogsvModel model = make_model(*params, eta, is_spot_measure != 0);
-  cudaStream_t st = current_stream();
-  ensure_pool_threshold();
-  DevBuf d_phi(st), d_psi(st), d_A(st), d_R(st);
-  B200SV_CUDA(d_phi.alloc(sizeof(cd) * P));
-  B200SV_CUDA(d_psi.alloc(sizeof(cd) * P));
-  B200SV_CUDA(d_A.alloc(sizeof(cd) * (size_t)P * N));
-  B200SV_CUDA(d_R.alloc(sizeof(cd) * (size_t)P * N));
-  B200SV_CUDA(cudaMemcpyAsync(d_phi.p, phi, sizeof(cd) * P, cudaMemcpyHostToDevice, st));
-  if (psi) B200SV_CUDA(cudaMemcpyAsync(d_psi.p, psi, sizeof(cd) * P, cudaMemcpyHostToDevice, st));
-  B200SV_CUDA(cudaMemcpyAsync(d_A.p, A, sizeof(cd) * (size_t)P * N, cudaMemcpyHostToDevice, st));
-  const cd* dpsi = psi ? d_psi.as<cd>() : nullptr;
-  if (N == 5)
-    logsv_ode_rhs_kernel<5><<<(P + 63) / 64, 64, 0, st>>>(d_phi.as<cd>(), dpsi, P, model, d_A.as<cd>(), d_R.as<cd>());
-  else
-    logsv_ode_rhs_kernel<3><<<(P + 63) / 64, 64, 0, st>>>(d_phi.as<cd>(), dpsi, P, model, d_A.as<cd>(), d_R.as<cd>());
-  if (int rc = launched("logsv_ode_rhs_kernel")) return rc;
-  B200SV_CUDA(cudaMemcpyAsync(rhs_out, d_R.p, sizeof(cd) * (size_t)P * N, cudaMemcpyDeviceToHost, st));
-  B200SV_CUDA(cudaStreamSynchronize(st));
-  return 0;
+  return host_call([&](cudaStream_t st) {
+    DevBuf<cd> d_phi(st), d_psi(st), d_A(st), d_R(st);
+    B200SV_CUDA(d_phi.upload(phi, P));
+    B200SV_CUDA(psi ? d_psi.upload(psi, P) : d_psi.alloc(P));
+    B200SV_CUDA(d_A.upload(A, (size_t)P * N));
+    B200SV_CUDA(d_R.alloc((size_t)P * N));
+    const cd* dpsi = psi ? d_psi.p : nullptr;
+    if (N == 5)
+      logsv_ode_rhs_kernel<5><<<(P + 63) / 64, 64, 0, st>>>(d_phi.p, dpsi, P, model, d_A.p, d_R.p);
+    else
+      logsv_ode_rhs_kernel<3><<<(P + 63) / 64, 64, 0, st>>>(d_phi.p, dpsi, P, model, d_A.p, d_R.p);
+    if (int rc = launched("logsv_ode_rhs_kernel")) return rc;
+    B200SV_CUDA(cudaMemcpyAsync(rhs_out, d_R.p, sizeof(cd) * (size_t)P * N, cudaMemcpyDeviceToHost, st));
+    return 0;
+  });
 }
 
 int b200sv_ode_rhs_dense(const double* A, int P, int n, const double* M, const double* L, const double* H, double* rhs_out) {
   B200SV_REQUIRE(A && M && L && H && rhs_out, "null pointer");
   B200SV_REQUIRE(P >= 1 && n >= 1 && n <= 16, "P >= 1, 1 <= n <= 16");
-  cudaStream_t st = current_stream();
-  ensure_pool_threshold();
-  DevBuf d_A(st), d_M(st), d_L(st), d_H(st), d_R(st);
-  B200SV_CUDA(d_A.alloc(sizeof(cd) * (size_t)P * n));
-  B200SV_CUDA(d_M.alloc(sizeof(cd) * (size_t)n * n * n));
-  B200SV_CUDA(d_L.alloc(sizeof(cd) * (size_t)n * n));
-  B200SV_CUDA(d_H.alloc(sizeof(cd) * n));
-  B200SV_CUDA(d_R.alloc(sizeof(cd) * (size_t)P * n));
-  B200SV_CUDA(cudaMemcpyAsync(d_A.p, A, sizeof(cd) * (size_t)P * n, cudaMemcpyHostToDevice, st));
-  B200SV_CUDA(cudaMemcpyAsync(d_M.p, M, sizeof(cd) * (size_t)n * n * n, cudaMemcpyHostToDevice, st));
-  B200SV_CUDA(cudaMemcpyAsync(d_L.p, L, sizeof(cd) * (size_t)n * n, cudaMemcpyHostToDevice, st));
-  B200SV_CUDA(cudaMemcpyAsync(d_H.p, H, sizeof(cd) * n, cudaMemcpyHostToDevice, st));
-  ode_rhs_dense_kernel<<<(P * n + 127) / 128, 128, 0, st>>>(d_A.as<cd>(), P, n, d_M.as<cd>(), d_L.as<cd>(), d_H.as<cd>(), d_R.as<cd>());
-  if (int rc = launched("ode_rhs_dense_kernel")) return rc;
-  B200SV_CUDA(cudaMemcpyAsync(rhs_out, d_R.p, sizeof(cd) * (size_t)P * n, cudaMemcpyDeviceToHost, st));
-  B200SV_CUDA(cudaStreamSynchronize(st));
-  return 0;
+  return host_call([&](cudaStream_t st) {
+    DevBuf<cd> d_A(st), d_M(st), d_L(st), d_H(st), d_R(st);
+    B200SV_CUDA(d_A.upload(A, (size_t)P * n));
+    B200SV_CUDA(d_M.upload(M, (size_t)n * n * n));
+    B200SV_CUDA(d_L.upload(L, (size_t)n * n));
+    B200SV_CUDA(d_H.upload(H, n));
+    B200SV_CUDA(d_R.alloc((size_t)P * n));
+    ode_rhs_dense_kernel<<<(P * n + 127) / 128, 128, 0, st>>>(d_A.p, P, n, d_M.p, d_L.p, d_H.p, d_R.p);
+    if (int rc = launched("ode_rhs_dense_kernel")) return rc;
+    B200SV_CUDA(cudaMemcpyAsync(rhs_out, d_R.p, sizeof(cd) * (size_t)P * n, cudaMemcpyDeviceToHost, st));
+    return 0;
+  });
 }
 
 // compute_logsv_a_mgf_grid(is_analytic=True): the semi-analytic branch over a transform grid (affine_expansion.py:388-470 -> :306-384)
@@ -2041,28 +1983,24 @@ int b200sv_logsv_mgf_grid_analytic(const double* phi, const double* psi, int P, 
   if (expansion_order != B200SV_ORDER_FIRST && expansion_order != B200SV_ORDER_SECOND) return fail(-4, "expansion_order not implemented");
   const int N = expansion_order == B200SV_ORDER_FIRST ? 3 : 5;
   const LogsvModel model = make_model(*params, 1.0, is_spot_measure != 0);      // eta is ignored on this branch (reference :340-348)
-  cudaStream_t st = current_stream();
-  ensure_pool_threshold();
-  DevBuf d_phi(st), d_psi(st), d_a0(st), d_a1(st), d_lm(st);
-  B200SV_CUDA(d_phi.alloc(sizeof(cd) * P));
-  B200SV_CUDA(d_psi.alloc(sizeof(cd) * P));
-  B200SV_CUDA(d_a0.alloc(sizeof(cd) * (size_t)P * N));
-  B200SV_CUDA(d_a1.alloc(sizeof(cd) * (size_t)P * N));
-  B200SV_CUDA(d_lm.alloc(sizeof(cd) * P));
-  B200SV_CUDA(cudaMemcpyAsync(d_phi.p, phi, sizeof(cd) * P, cudaMemcpyHostToDevice, st));
-  if (psi) B200SV_CUDA(cudaMemcpyAsync(d_psi.p, psi, sizeof(cd) * P, cudaMemcpyHostToDevice, st));
-  B200SV_CUDA(cudaMemcpyAsync(d_a0.p, a_inout, sizeof(cd) * (size_t)P * N, cudaMemcpyHostToDevice, st));
-  const cd* dpsi = psi ? d_psi.as<cd>() : nullptr;
-  const double y = params->sigma0 - params->theta;
-  if (N == 5)
-    logsv_mgf_analytic_kernel<5><<<(P + 63) / 64, 64, 0, st>>>(d_phi.as<cd>(), dpsi, P, model, dtau, year_days, d_a0.as<cd>(), d_a1.as<cd>(), d_lm.as<cd>(), y);
-  else
-    logsv_mgf_analytic_kernel<3><<<(P + 63) / 64, 64, 0, st>>>(d_phi.as<cd>(), dpsi, P, model, dtau, year_days, d_a0.as<cd>(), d_a1.as<cd>(), d_lm.as<cd>(), y);
-  if (int rc = launched("logsv_mgf_analytic_kernel")) return rc;
-  B200SV_CUDA(cudaMemcpyAsync(a_inout, d_a1.p, sizeof(cd) * (size_t)P * N, cudaMemcpyDeviceToHost, st));
-  B200SV_CUDA(cudaMemcpyAsync(log_mgf_out, d_lm.p, sizeof(cd) * P, cudaMemcpyDeviceToHost, st));
-  B200SV_CUDA(cudaStreamSynchronize(st));
-  return 0;
+  return host_call([&](cudaStream_t st) {
+    DevBuf<cd> d_phi(st), d_psi(st), d_a0(st), d_a1(st), d_lm(st);
+    B200SV_CUDA(d_phi.upload(phi, P));
+    B200SV_CUDA(psi ? d_psi.upload(psi, P) : d_psi.alloc(P));
+    B200SV_CUDA(d_a0.upload(a_inout, (size_t)P * N));
+    B200SV_CUDA(d_a1.alloc((size_t)P * N));
+    B200SV_CUDA(d_lm.alloc(P));
+    const cd* dpsi = psi ? d_psi.p : nullptr;
+    const double y = params->sigma0 - params->theta;
+    if (N == 5)
+      logsv_mgf_analytic_kernel<5><<<(P + 63) / 64, 64, 0, st>>>(d_phi.p, dpsi, P, model, dtau, year_days, d_a0.p, d_a1.p, d_lm.p, y);
+    else
+      logsv_mgf_analytic_kernel<3><<<(P + 63) / 64, 64, 0, st>>>(d_phi.p, dpsi, P, model, dtau, year_days, d_a0.p, d_a1.p, d_lm.p, y);
+    if (int rc = launched("logsv_mgf_analytic_kernel")) return rc;
+    B200SV_CUDA(cudaMemcpyAsync(a_inout, d_a1.p, sizeof(cd) * (size_t)P * N, cudaMemcpyDeviceToHost, st));
+    B200SV_CUDA(cudaMemcpyAsync(log_mgf_out, d_lm.p, sizeof(cd) * P, cudaMemcpyDeviceToHost, st));
+    return 0;
+  });
 }
 
 // compute_logsv_a_mgf_grid(is_stiff_solver=True): SciPy's BDF control law per grid point (affine_expansion.py:229-303)
@@ -2073,59 +2011,50 @@ int b200sv_logsv_mgf_grid_bdf(const double* phi, const double* psi, int P, doubl
   if (expansion_order != B200SV_ORDER_FIRST && expansion_order != B200SV_ORDER_SECOND) return fail(-4, "expansion_order not implemented");
   const int N = expansion_order == B200SV_ORDER_FIRST ? 3 : 5;
   const LogsvModel model = make_model(*params, eta, is_spot_measure != 0);
-  cudaStream_t st = current_stream();
-  ensure_pool_threshold();
-  DevBuf d_phi(st), d_psi(st), d_a0(st), d_a1(st), d_lm(st);
-  B200SV_CUDA(d_phi.alloc(sizeof(cd) * P));
-  B200SV_CUDA(d_psi.alloc(sizeof(cd) * P));
-  B200SV_CUDA(d_a0.alloc(sizeof(cd) * (size_t)P * N));
-  B200SV_CUDA(d_a1.alloc(sizeof(cd) * (size_t)P * N));
-  B200SV_CUDA(d_lm.alloc(sizeof(cd) * P));
-  B200SV_CUDA(cudaMemcpyAsync(d_phi.p, phi, sizeof(cd) * P, cudaMemcpyHostToDevice, st));
-  if (psi) B200SV_CUDA(cudaMemcpyAsync(d_psi.p, psi, sizeof(cd) * P, cudaMemcpyHostToDevice, st));
-  B200SV_CUDA(cudaMemcpyAsync(d_a0.p, a_inout, sizeof(cd) * (size_t)P * N, cudaMemcpyHostToDevice, st));
-  const cd* dpsi = psi ? d_psi.as<cd>() : nullptr;
-  const double y = params->sigma0 - params->theta;
-  if (N == 5)
-    logsv_mgf_bdf_kernel<5><<<(P + 63) / 64, 64, 0, st>>>(d_phi.as<cd>(), dpsi, P, model, dtau, d_a0.as<cd>(), d_a1.as<cd>(), d_lm.as<cd>(), y, nullptr);
-  else
-    logsv_mgf_bdf_kernel<3><<<(P + 63) / 64, 64, 0, st>>>(d_phi.as<cd>(), dpsi, P, model, dtau, d_a0.as<cd>(), d_a1.as<cd>(), d_lm.as<cd>(), y, nullptr);
-  if (int rc = launched("logsv_mgf_bdf_kernel")) return rc;
-  B200SV_CUDA(cudaMemcpyAsync(a_inout, d_a1.p, sizeof(cd) * (size_t)P * N, cudaMemcpyDeviceToHost, st));
-  B200SV_CUDA(cudaMemcpyAsync(log_mgf_out, d_lm.p, sizeof(cd) * P, cudaMemcpyDeviceToHost, st));
-  B200SV_CUDA(cudaStreamSynchronize(st));
-  return 0;
+  return host_call([&](cudaStream_t st) {
+    DevBuf<cd> d_phi(st), d_psi(st), d_a0(st), d_a1(st), d_lm(st);
+    B200SV_CUDA(d_phi.upload(phi, P));
+    B200SV_CUDA(psi ? d_psi.upload(psi, P) : d_psi.alloc(P));
+    B200SV_CUDA(d_a0.upload(a_inout, (size_t)P * N));
+    B200SV_CUDA(d_a1.alloc((size_t)P * N));
+    B200SV_CUDA(d_lm.alloc(P));
+    const cd* dpsi = psi ? d_psi.p : nullptr;
+    const double y = params->sigma0 - params->theta;
+    if (N == 5)
+      logsv_mgf_bdf_kernel<5><<<(P + 63) / 64, 64, 0, st>>>(d_phi.p, dpsi, P, model, dtau, d_a0.p, d_a1.p, d_lm.p, y, nullptr);
+    else
+      logsv_mgf_bdf_kernel<3><<<(P + 63) / 64, 64, 0, st>>>(d_phi.p, dpsi, P, model, dtau, d_a0.p, d_a1.p, d_lm.p, y, nullptr);
+    if (int rc = launched("logsv_mgf_bdf_kernel")) return rc;
+    B200SV_CUDA(cudaMemcpyAsync(a_inout, d_a1.p, sizeof(cd) * (size_t)P * N, cudaMemcpyDeviceToHost, st));
+    B200SV_CUDA(cudaMemcpyAsync(log_mgf_out, d_lm.p, sizeof(cd) * P, cudaMemcpyDeviceToHost, st));
+    return 0;
+  });
 }
 
 int b200sv_heston_mgf_grid(const double* phi, const double* psi, int P, double dtau, double* a_inout, double* b_inout,
                            const b200sv_heston_params* params, double* log_mgf_out) {
   B200SV_REQUIRE(phi && a_inout && b_inout && params && log_mgf_out, "null pointer");
   B200SV_REQUIRE(P >= 1 && dtau > 0.0, "P >= 1, dtau > 0");
-  cudaStream_t st = current_stream();
-  ensure_pool_threshold();
-  DevBuf d_phi(st), d_psi(st), d_dt(st), d_a(st), d_b(st), d_a1(st), d_b1(st), d_lm(st);
-  B200SV_CUDA(d_phi.alloc(sizeof(cd) * P));
-  B200SV_CUDA(d_psi.alloc(sizeof(cd) * P));
-  B200SV_CUDA(d_dt.alloc(sizeof(double)));
-  B200SV_CUDA(d_a.alloc(sizeof(cd) * P));
-  B200SV_CUDA(d_b.alloc(sizeof(cd) * P));
-  B200SV_CUDA(d_a1.alloc(sizeof(cd) * P));
-  B200SV_CUDA(d_b1.alloc(sizeof(cd) * P));
-  B200SV_CUDA(d_lm.alloc(sizeof(cd) * P));
-  B200SV_CUDA(cudaMemcpyAsync(d_phi.p, phi, sizeof(cd) * P, cudaMemcpyHostToDevice, st));
-  if (psi) B200SV_CUDA(cudaMemcpyAsync(d_psi.p, psi, sizeof(cd) * P, cudaMemcpyHostToDevice, st));
-  B200SV_CUDA(cudaMemcpyAsync(d_dt.p, &dtau, sizeof(double), cudaMemcpyHostToDevice, st));
-  B200SV_CUDA(cudaMemcpyAsync(d_a.p, a_inout, sizeof(cd) * P, cudaMemcpyHostToDevice, st));
-  B200SV_CUDA(cudaMemcpyAsync(d_b.p, b_inout, sizeof(cd) * P, cudaMemcpyHostToDevice, st));
-  const int tpb = mgf_block_threads(P), nb = (P + tpb - 1) / tpb;
-  heston_mgf_kernel<<<nb, tpb, 0, st>>>(d_phi.as<cd>(), psi ? d_psi.as<cd>() : nullptr, P, 1, d_dt.as<double>(), *params,
-                                        d_a.as<cd>(), d_b.as<cd>(), d_a1.as<cd>(), d_b1.as<cd>(), d_lm.as<cd>());
-  if (int rc = launched("heston_mgf_kernel")) return rc;
-  B200SV_CUDA(cudaMemcpyAsync(a_inout, d_a1.p, sizeof(cd) * P, cudaMemcpyDeviceToHost, st));
-  B200SV_CUDA(cudaMemcpyAsync(b_inout, d_b1.p, sizeof(cd) * P, cudaMemcpyDeviceToHost, st));
-  B200SV_CUDA(cudaMemcpyAsync(log_mgf_out, d_lm.p, sizeof(cd) * P, cudaMemcpyDeviceToHost, st));
-  B200SV_CUDA(cudaStreamSynchronize(st));
-  return 0;
+  return host_call([&](cudaStream_t st) {
+    DevBuf<cd> d_phi(st), d_psi(st), d_a(st), d_b(st), d_a1(st), d_b1(st), d_lm(st);
+    DevBuf<double> d_dt(st);
+    B200SV_CUDA(d_phi.upload(phi, P));
+    B200SV_CUDA(psi ? d_psi.upload(psi, P) : d_psi.alloc(P));
+    B200SV_CUDA(d_dt.upload(&dtau, 1));
+    B200SV_CUDA(d_a.upload(a_inout, P));
+    B200SV_CUDA(d_b.upload(b_inout, P));
+    B200SV_CUDA(d_a1.alloc(P));
+    B200SV_CUDA(d_b1.alloc(P));
+    B200SV_CUDA(d_lm.alloc(P));
+    const int tpb = mgf_block_threads(P), nb = (P + tpb - 1) / tpb;
+    heston_mgf_kernel<<<nb, tpb, 0, st>>>(d_phi.p, psi ? d_psi.p : nullptr, P, 1, d_dt.p, *params,
+                                          d_a.p, d_b.p, d_a1.p, d_b1.p, d_lm.p);
+    if (int rc = launched("heston_mgf_kernel")) return rc;
+    B200SV_CUDA(cudaMemcpyAsync(a_inout, d_a1.p, sizeof(cd) * P, cudaMemcpyDeviceToHost, st));
+    B200SV_CUDA(cudaMemcpyAsync(b_inout, d_b1.p, sizeof(cd) * P, cudaMemcpyDeviceToHost, st));
+    B200SV_CUDA(cudaMemcpyAsync(log_mgf_out, d_lm.p, sizeof(cd) * P, cudaMemcpyDeviceToHost, st));
+    return 0;
+  });
 }
 
 int b200sv_fourier_vanilla(const double* log_mgf, const double* phi, int P, double forward, const double* strikes,
@@ -2136,22 +2065,20 @@ int b200sv_fourier_vanilla(const double* log_mgf, const double* phi, int P, doub
   if (int rc = check_fourier_types(types, J, spot)) return rc;
   std::vector<StrikeSpec> ss(J);
   for (int j = 0; j < J; ++j) ss[j] = StrikeSpec{strikes[j], forward, discfactor, (int)types[j], 0, 1.0, 0};
-  cudaStream_t st = current_stream();
-  ensure_pool_threshold();
-  DevBuf d_phi(st), d_lm(st), d_ss(st), d_pr(st);
-  B200SV_CUDA(d_phi.alloc(sizeof(cd) * P));
-  B200SV_CUDA(d_lm.alloc(sizeof(cd) * P));
-  B200SV_CUDA(d_ss.alloc(sizeof(StrikeSpec) * J));
-  B200SV_CUDA(d_pr.alloc(sizeof(double) * J));
-  B200SV_CUDA(cudaMemcpyAsync(d_phi.p, phi, sizeof(cd) * P, cudaMemcpyHostToDevice, st));
-  B200SV_CUDA(cudaMemcpyAsync(d_lm.p, log_mgf, sizeof(cd) * P, cudaMemcpyHostToDevice, st));
-  B200SV_CUDA(cudaMemcpyAsync(d_ss.p, ss.data(), sizeof(StrikeSpec) * J, cudaMemcpyHostToDevice, st));
-  fourier_vanilla_kernel<<<J, kFourierThreads, 0, st>>>(d_lm.as<cd>(), d_phi.as<cd>(), P, d_ss.as<StrikeSpec>(), spot ? 1 : 0,
-                                                        all_half_re(phi, P) ? 1 : 0, d_pr.as<double>());
-  if (int rc = launched("fourier_vanilla_kernel")) return rc;
-  B200SV_CUDA(cudaMemcpyAsync(prices_out, d_pr.p, sizeof(double) * J, cudaMemcpyDeviceToHost, st));
-  B200SV_CUDA(cudaStreamSynchronize(st));
-  return 0;
+  return host_call([&](cudaStream_t st) {
+    DevBuf<cd> d_phi(st), d_lm(st);
+    DevBuf<StrikeSpec> d_ss(st);
+    DevBuf<double> d_pr(st);
+    B200SV_CUDA(d_phi.upload(phi, P));
+    B200SV_CUDA(d_lm.upload(log_mgf, P));
+    B200SV_CUDA(d_ss.upload(ss.data(), J));
+    B200SV_CUDA(d_pr.alloc(J));
+    fourier_vanilla_kernel<<<J, kFourierThreads, 0, st>>>(d_lm.p, d_phi.p, P, d_ss.p, spot ? 1 : 0,
+                                                          all_half_re(phi, P) ? 1 : 0, d_pr.p);
+    if (int rc = launched("fourier_vanilla_kernel")) return rc;
+    B200SV_CUDA(cudaMemcpyAsync(prices_out, d_pr.p, sizeof(double) * J, cudaMemcpyDeviceToHost, st));
+    return 0;
+  });
 }
 
 /* slice_pricer_with_mgf_grid_with_gamma (utils/mgf_pricer.py:273-320) on caller-supplied log-MGF / transform grids: 'C' / 'P' under the spot
@@ -2166,42 +2093,38 @@ int b200sv_fourier_gamma(const double* log_mgf, const double* phi, int P, double
     if (types[j] != B200SV_CALL && types[j] != B200SV_PUT) return fail(-5, "not implemented");
     ss[j] = StrikeSpec{strikes[j], forward, normalizer, (int)types[j], 0, gamma_forward, 0};
   }
-  cudaStream_t st = current_stream();
-  ensure_pool_threshold();
-  DevBuf d_phi(st), d_lm(st), d_ss(st), d_pr(st);
-  B200SV_CUDA(d_phi.alloc(sizeof(cd) * P));
-  B200SV_CUDA(d_lm.alloc(sizeof(cd) * P));
-  B200SV_CUDA(d_ss.alloc(sizeof(StrikeSpec) * J));
-  B200SV_CUDA(d_pr.alloc(sizeof(double) * J));
-  B200SV_CUDA(cudaMemcpyAsync(d_phi.p, phi, sizeof(cd) * P, cudaMemcpyHostToDevice, st));
-  B200SV_CUDA(cudaMemcpyAsync(d_lm.p, log_mgf, sizeof(cd) * P, cudaMemcpyHostToDevice, st));
-  B200SV_CUDA(cudaMemcpyAsync(d_ss.p, ss.data(), sizeof(StrikeSpec) * J, cudaMemcpyHostToDevice, st));
-  fourier_gamma_kernel<<<J, kFourierThreads, 0, st>>>(d_lm.as<cd>(), d_phi.as<cd>(), P, d_ss.as<StrikeSpec>(), risk_premia_gamma, d_pr.as<double>());
-  if (int rc = launched("fourier_gamma_kernel")) return rc;
-  B200SV_CUDA(cudaMemcpyAsync(prices_out, d_pr.p, sizeof(double) * J, cudaMemcpyDeviceToHost, st));
-  B200SV_CUDA(cudaStreamSynchronize(st));
-  return 0;
+  return host_call([&](cudaStream_t st) {
+    DevBuf<cd> d_phi(st), d_lm(st);
+    DevBuf<StrikeSpec> d_ss(st);
+    DevBuf<double> d_pr(st);
+    B200SV_CUDA(d_phi.upload(phi, P));
+    B200SV_CUDA(d_lm.upload(log_mgf, P));
+    B200SV_CUDA(d_ss.upload(ss.data(), J));
+    B200SV_CUDA(d_pr.alloc(J));
+    fourier_gamma_kernel<<<J, kFourierThreads, 0, st>>>(d_lm.p, d_phi.p, P, d_ss.p, risk_premia_gamma, d_pr.p);
+    if (int rc = launched("fourier_gamma_kernel")) return rc;
+    B200SV_CUDA(cudaMemcpyAsync(prices_out, d_pr.p, sizeof(double) * J, cudaMemcpyDeviceToHost, st));
+    return 0;
+  });
 }
 
 // shared driver of the generic sums
 static int fourier_sum_host(const double* log_mgf, const double* grid, int P, const std::vector<SumSpec>& specs, int mode, int all_calls,
                             double* out) {
   const int J = (int)specs.size();
-  cudaStream_t st = current_stream();
-  ensure_pool_threshold();
-  DevBuf d_g(st), d_lm(st), d_ss(st), d_pr(st);
-  B200SV_CUDA(d_g.alloc(sizeof(cd) * P));
-  B200SV_CUDA(d_lm.alloc(sizeof(cd) * P));
-  B200SV_CUDA(d_ss.alloc(sizeof(SumSpec) * J));
-  B200SV_CUDA(d_pr.alloc(sizeof(double) * J));
-  B200SV_CUDA(cudaMemcpyAsync(d_g.p, grid, sizeof(cd) * P, cudaMemcpyHostToDevice, st));
-  B200SV_CUDA(cudaMemcpyAsync(d_lm.p, log_mgf, sizeof(cd) * P, cudaMemcpyHostToDevice, st));
-  B200SV_CUDA(cudaMemcpyAsync(d_ss.p, specs.data(), sizeof(SumSpec) * J, cudaMemcpyHostToDevice, st));
-  fourier_sum_kernel<<<J, kFourierThreads, 0, st>>>(d_lm.as<cd>(), d_g.as<cd>(), P, d_ss.as<SumSpec>(), mode, all_calls, d_pr.as<double>());
-  if (int rc = launched("fourier_sum_kernel")) return rc;
-  B200SV_CUDA(cudaMemcpyAsync(out, d_pr.p, sizeof(double) * J, cudaMemcpyDeviceToHost, st));
-  B200SV_CUDA(cudaStreamSynchronize(st));
-  return 0;
+  return host_call([&](cudaStream_t st) {
+    DevBuf<cd> d_g(st), d_lm(st);
+    DevBuf<SumSpec> d_ss(st);
+    DevBuf<double> d_pr(st);
+    B200SV_CUDA(d_g.upload(grid, P));
+    B200SV_CUDA(d_lm.upload(log_mgf, P));
+    B200SV_CUDA(d_ss.upload(specs.data(), J));
+    B200SV_CUDA(d_pr.alloc(J));
+    fourier_sum_kernel<<<J, kFourierThreads, 0, st>>>(d_lm.p, d_g.p, P, d_ss.p, mode, all_calls, d_pr.p);
+    if (int rc = launched("fourier_sum_kernel")) return rc;
+    B200SV_CUDA(cudaMemcpyAsync(out, d_pr.p, sizeof(double) * J, cudaMemcpyDeviceToHost, st));
+    return 0;
+  });
 }
 
 int b200sv_fourier_qvar(const double* log_mgf, const double* psi, int P, double ttm, const double* strikes, const int8_t* types, int J,

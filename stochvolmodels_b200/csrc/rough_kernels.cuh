@@ -188,7 +188,7 @@ static int launch_rough_n(double* ls, double* vol, double* qv, const double* Z0,
     rough_logsv_kernel<N, kGaussF64><<<g.blocks, g.threads, 0, st>>>(ls, vol, qv, Z0, Z1, S, P, c, seed, (unsigned long long)path_offset);
   else
     rough_logsv_kernel<N, kGaussF32><<<g.blocks, g.threads, 0, st>>>(ls, vol, qv, Z0, Z1, S, P, c, seed, (unsigned long long)path_offset);
-  return check_launch("rough_logsv_kernel");
+  return launched("rough_logsv_kernel");
 }
 
 static int launch_rough(int n, double* ls, double* vol, double* qv, const double* Z0, const double* Z1, int S, long long P, const RoughConsts& c,
@@ -226,71 +226,33 @@ static int rough_chain_host(const b200sv_logsv_params* params, int B, int n, con
     Smax = std::max(Smax, nsteps[m]);
   }
   B200SV_REQUIRE(!Z0 || z_rows >= Smax, "Z0 / Z1 have fewer rows than the longest grid");
-  const int Jtot = offsets[M] - offsets[0], Jalloc = std::max(Jtot, 1);
-  cudaStream_t st = current_stream();
-  ensure_pool_threshold();
   const size_t P = (size_t)nb_path;
-  double *d_state = nullptr, *d_z = nullptr, *d_strikes = nullptr, *d_out = nullptr, *d_mom = nullptr, *d_sums = nullptr;
-  int8_t* d_types = nullptr;
-  B200SV_CUDA(cudaMallocAsync(&d_state, sizeof(double) * (size_t)(n + 2) * P, st));
-  if (Z0) {
-    B200SV_CUDA(cudaMallocAsync(&d_z, sizeof(double) * 2 * (size_t)Smax * P, st));
-    B200SV_CUDA(cudaMemcpyAsync(d_z, Z0, sizeof(double) * (size_t)Smax * P, cudaMemcpyHostToDevice, st));
-    B200SV_CUDA(cudaMemcpyAsync(d_z + (size_t)Smax * P, Z1, sizeof(double) * (size_t)Smax * P, cudaMemcpyHostToDevice, st));
-  }
-  B200SV_CUDA(cudaMallocAsync(&d_strikes, sizeof(double) * Jalloc, st));
-  B200SV_CUDA(cudaMallocAsync(&d_types, Jalloc, st));
-  const size_t out_stride = (size_t)3 * Jalloc;
-  B200SV_CUDA(cudaMallocAsync(&d_out, sizeof(double) * out_stride * B, st));
-  B200SV_CUDA(cudaMallocAsync(&d_mom, sizeof(double) * 2, st));
-  B200SV_CUDA(cudaMallocAsync(&d_sums, sizeof(double) * 3 * Jalloc, st));
-  if (Jtot > 0) {
-    B200SV_CUDA(cudaMemcpyAsync(d_strikes, strikes + offsets[0], sizeof(double) * Jtot, cudaMemcpyHostToDevice, st));
-    B200SV_CUDA(cudaMemcpyAsync(d_types, types + offsets[0], Jtot, cudaMemcpyHostToDevice, st));
-  }
-  double *d_ls = d_state, *d_vol = d_state + P, *d_qv = d_state + (size_t)(n + 1) * P;
-  int rc = 0;
-  for (int b = 0; b < B && rc == 0; ++b) {
-    double* out_b = d_out + out_stride * b;
-    for (int m = 0; m < M && rc == 0; ++m) {
-      const RoughConsts c = make_rough_consts(params[b], n, weights + (size_t)b * n, nodes + (size_t)b * n, hs[m]);
-      rc = launch_rough(n, d_ls, d_vol, d_qv, d_z, d_z ? d_z + (size_t)Smax * P : nullptr, nsteps[m], nb_path, c, seed, 0, g, st);
-      if (rc) break;
-      if (states_out) {
-        cudaError_t e = cudaMemcpyAsync(states_out + (size_t)m * (n + 2) * P, d_state, sizeof(double) * (size_t)(n + 2) * P, cudaMemcpyDeviceToHost, st);
-        if (e != cudaSuccess) rc = fail(-2, std::string("D2H: ") + cudaGetErrorString(e));
-      }
-      const int J = offsets[m + 1] - offsets[m], jo = offsets[m] - offsets[0];
-      if (J == 0 || rc) continue;
-      rc = b200sv_dev_spot_moments(d_ls, nb_path, forwards[m], d_mom, st);
-      if (rc == 0)
-        rc = launch_payoff_t<double>(d_ls, d_qv, nb_path, ttms[m], forwards[m], d_strikes + jo, d_types + jo, J, variable_type,
-                                     payoff_kinds(types + offsets[m], J), d_mom, d_sums, st);
-      if (rc) break;
-      // the reference hands (1, nb_path)-shaped arrays to compute_mc_vars_payoff, whose "/ sqrt(x0.shape[0])" is then "/ 1":
-      // this route's std errors are discfactor * nanstd(payoff) (total_paths = 1)
-      const IvolSpec iv{d_strikes + jo, d_types + jo, forwards[m], ttms[m], ivols_out ? out_b + 2 * Jalloc + jo : nullptr};
-      payoff_finalize_kernel<<<(J + 127) / 128, 128, 0, st>>>(d_sums, J, discfactors[m], 1.0, out_b + jo, out_b + Jalloc + jo, P2pGather{}, iv);
-      rc = check_launch("payoff_finalize_kernel");
+  return host_call([&](cudaStream_t st) {
+    DevBuf<double> d_state(st), d_z(st);
+    ChainPayoffs pay(st, M, ttms, forwards, discfactors, offsets, types, variable_type, B, ivols_out != nullptr);
+    B200SV_CUDA(d_state.alloc((size_t)(n + 2) * P));
+    if (Z0) {
+      B200SV_CUDA(d_z.alloc(2 * (size_t)Smax * P));
+      B200SV_CUDA(cudaMemcpyAsync(d_z.p, Z0, sizeof(double) * (size_t)Smax * P, cudaMemcpyHostToDevice, st));
+      B200SV_CUDA(cudaMemcpyAsync(d_z.p + (size_t)Smax * P, Z1, sizeof(double) * (size_t)Smax * P, cudaMemcpyHostToDevice, st));
     }
-  }
-  for (int b = 0; b < B && rc == 0 && Jtot > 0; ++b) {
-    const double* out_b = d_out + out_stride * b;
-    cudaError_t e = cudaMemcpyAsync(prices_out + (size_t)b * Jtot, out_b, sizeof(double) * Jtot, cudaMemcpyDeviceToHost, st);
-    if (e == cudaSuccess) e = cudaMemcpyAsync(stderr_out + (size_t)b * Jtot, out_b + Jalloc, sizeof(double) * Jtot, cudaMemcpyDeviceToHost, st);
-    if (e == cudaSuccess && ivols_out) e = cudaMemcpyAsync(ivols_out + (size_t)b * Jtot, out_b + 2 * Jalloc, sizeof(double) * Jtot, cudaMemcpyDeviceToHost, st);
-    if (e != cudaSuccess) rc = fail(-2, std::string("D2H: ") + cudaGetErrorString(e));
-  }
-  cudaFreeAsync(d_state, st);
-  if (d_z) cudaFreeAsync(d_z, st);
-  cudaFreeAsync(d_strikes, st);
-  cudaFreeAsync(d_types, st);
-  cudaFreeAsync(d_out, st);
-  cudaFreeAsync(d_mom, st);
-  cudaFreeAsync(d_sums, st);
-  cudaError_t e = cudaStreamSynchronize(st);
-  if (rc == 0 && e != cudaSuccess) rc = fail(-2, std::string("sync: ") + cudaGetErrorString(e));
-  return rc;
+    if (int rc = pay.alloc(strikes)) return rc;
+    double *d_ls = d_state.p, *d_vol = d_state.p + P, *d_qv = d_state.p + (size_t)(n + 1) * P;
+    for (int b = 0; b < B; ++b)
+      for (int m = 0; m < M; ++m) {
+        const RoughConsts c = make_rough_consts(params[b], n, weights + (size_t)b * n, nodes + (size_t)b * n, hs[m]);
+        if (int rc = launch_rough(n, d_ls, d_vol, d_qv, d_z.p, Z0 ? d_z.p + (size_t)Smax * P : nullptr, nsteps[m], nb_path, c, seed, 0, g, st))
+          return rc;
+        if (states_out)
+          B200SV_CUDA(cudaMemcpyAsync(states_out + (size_t)m * (n + 2) * P, d_state.p, sizeof(double) * (size_t)(n + 2) * P, cudaMemcpyDeviceToHost, st));
+        if (offsets[m + 1] == offsets[m]) continue;
+        if (int rc = b200sv_dev_spot_moments(d_ls, nb_path, forwards[m], pay.d_mom.p, st)) return rc;
+        // the reference hands (1, nb_path)-shaped arrays to compute_mc_vars_payoff, whose "/ sqrt(x0.shape[0])" is then "/ 1":
+        // this route's std errors are discfactor * nanstd(payoff) (total_paths = 1)
+        if (int rc = pay.run(b, m, d_ls, d_qv, nb_path, false, 1.0, st)) return rc;
+      }
+    return pay.copy_back(prices_out, stderr_out, ivols_out, st);
+  });
 }
 
 }  // namespace b200sv
